@@ -2,7 +2,7 @@
 """bench.py — headline benchmark of the hot path (BASELINE.json: "DDH-GMRES solve time & GDOF/s operator apply at 1/2/4/8
 B200 vs %HBM roofline").
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--dump-outputs DIR]
 
 value / e2e / roofline  (BASELINE configs[1]): operator apply on a synthetic structured 1024x1024 quad mesh, n_basis 5
     (degree 4): one "step" is one Helmholtz composite action (stiffness + weighted mass on u and v, boundary face mass) on
@@ -17,6 +17,8 @@ value / e2e / roofline  (BASELINE configs[1]): operator apply on a synthetic str
 `--impl reference` times the CPU restatement of the reference's kernels (oracle/, OpenMP over all host cores; the reference
 has no host-only build, SURVEY R6) on the SAME 1024^2 workload, index data from the oracle's own closed-form numpy setup (the
 product library is not loaded). Prints ONE JSON line on rank 0.
+`--dump-outputs DIR` writes y = A [u; v] of the last timed step to DIR (see dump_outputs), so that two builds can be compared
+output for output: the inputs depend on nothing but the arguments.
 """
 import argparse
 import json
@@ -34,10 +36,33 @@ sys.path.insert(0, ROOT)
 
 METRIC = "helmholtz_operator_apply_gdofs"
 UNIT = "GDOF/s"
+DUMP_VALUES = 1 << 22  # --dump-outputs: float64 entries of y written at most, over all ranks (32 MiB)
 
 
 def coef(x, y):
     return 1.0 + 0.5 * np.sin(np.pi * x) * np.cos(np.pi * y)
+
+
+def dump_sample(n, world):
+    """positions kept by --dump-outputs in a vector of n entries: all of them when n fits this rank's share of DUMP_VALUES,
+    else one entry drawn from each of that many equal strata with a fixed seed (a function of n and world only)"""
+    k = DUMP_VALUES // world
+    if n <= k:
+        return np.arange(n, dtype=np.int64)
+    edges = np.arange(k + 1, dtype=np.int64) * n // k
+    return edges[:-1] + np.random.default_rng(2024).integers(0, np.diff(edges))
+
+
+def dump_outputs(out_dir, take, n, rank, world):
+    """y = A [u; v] as the caller of the timed apply receives it, as DIR/helmholtz_y.npy (float64): the entries dump_sample(n, world)
+    picks, in increasing position. take(idx) returns y[idx] as a numpy array. N > 1: one file per rank (helmholtz_y_rank<r>.npy),
+    DUMP_VALUES entries in all."""
+    idx = dump_sample(n, world)
+    name = "helmholtz_y%s.npy" % ("_rank%d" % rank if world > 1 else "")
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, name), np.asarray(take(idx), np.float64))
+    return {"dir": out_dir, "file": name, "entries": len(idx), "of": n,
+            "positions": "bench.dump_sample(%d, %d): one entry per stratum, seed 2024" % (n, world) if len(idx) < n else "all"}
 
 
 def workload(args):
@@ -133,16 +158,16 @@ def time_cpu_port(nx, nb, omega, steps, warmup):
         A.action(x)
     t0 = time.perf_counter()
     for _ in range(steps):
-        A.action(x)
+        y = A.action(x)
     dt = (time.perf_counter() - t0) / steps
-    return 2 * ndof / dt / 1e9, dt, O.max_threads(), ndof
+    return 2 * ndof / dt / 1e9, dt, O.max_threads(), ndof, y
 
 
 def run_reference_arm(args):
     rank = int(os.environ.get("RANK", "0"))
     if rank != 0:
         return
-    val, dt, cores, ndof = time_cpu_port(args.nx, args.nb, args.omega, args.steps, args.warmup)
+    val, dt, cores, ndof, y = time_cpu_port(args.nx, args.nb, args.omega, args.steps, args.warmup)
     sample = "the full uniform_rect(%d) n_basis %d workload (one slab), %d applies of %.3f s, OpenMP %d threads" % (
         args.nx, args.nb, args.steps, dt, cores)
     line = {"impl": "reference", "metric": METRIC, "value": val, "unit": UNIT, "n_gpus": args.gpus, "steps": args.steps,
@@ -155,14 +180,17 @@ def run_reference_arm(args):
             "note": "the reference has no host-only build (all operator bodies are __device__ lambdas, SURVEY R6); this arm is the CPU "
                     "restatement in oracle/oracle.c on one 1024^2 slab (one CPU run whatever N is), index data from "
                     "oracle/setup_np.py:uniform_rect_closed_form (pinned to the reference's own 1024^2 hashes); libcuddh_b200.so is not loaded"}
+    if args.dump_outputs:  # same x as rank 0 of the GPU path, same positions: comparable file for file with a single-GPU dump
+        line["dump_outputs"] = dump_outputs(args.dump_outputs, lambda idx: y[idx], y.size, 0, 1)
     print(json.dumps(line))
 
 
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=20)
-    ap.add_argument("--warmup", type=int, default=3)
+    ap.add_argument("--steps", type=int, default=20, help="timed applies of the headline (device-resident) loop; the end-to-end leg runs "
+                    "max(6, min(steps, 12)) requests and the roofline kernel timing max(steps, 20) launches")
+    ap.add_argument("--warmup", type=int, default=3, help="untimed applies before the timed loop (at least 3)")
     ap.add_argument("--impl", default="ours")
     ap.add_argument("--nx", type=int, default=1024)
     ap.add_argument("--nb", type=int, default=5)
@@ -173,7 +201,11 @@ def main():
     ap.add_argument("--ddh-solve-nx", type=int, default=512)
     ap.add_argument("--ddh-ho-nx", type=int, default=512, help="mesh of the scaled-down high-order (configs[4]) DDH action")
     ap.add_argument("--ddh-box-seconds", type=float, default=45.0, help="time box of the GMRES(30) restart cycle at config 3")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write y = A [u; v] of the last timed step to DIR/*.npy (a fixed, seeded sample of at most %d entries over all ranks)" % DUMP_VALUES)
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     args.warmup = max(args.warmup, 3)
 
     if args.impl == "reference":
@@ -234,6 +266,10 @@ def main():
     launches = cb.launch_count() - l0
     ms_step = max_over_ranks(e0.elapsed_time(e1)) / K
     value = 2.0 * ndof * world / (ms_step * 1e-3) / 1e9
+    # y still holds the last timed step's result (the legs below overwrite it)
+    dumped = None
+    if args.dump_outputs:
+        dumped = dump_outputs(args.dump_outputs, lambda idx: y[torch.as_tensor(idx, device=y.device)].cpu().numpy(), y.numel(), rank, world)
 
     # ---- end to end through the public API with HOST buffers: every step copies its [u; v] from pinned host memory, applies
     # the operator and reads the result back to the host. Consecutive steps are independent requests, so they are
@@ -296,6 +332,8 @@ def main():
             "gpu_launches": int(launches), "clocks": sampler.summary() if sampler else None}
     if world > 1:
         line["exchange"] = slab.exchange_info()
+    if dumped:
+        line["dump_outputs"] = dumped
 
     # ---- roofline of the dominant kernel, timed alone with CUDA events on its stream: the fused Helmholtz volume kernel
     # (S - omega^2 M on u and v; > 90 % of the step). Algorithmic bytes = SURVEY §8(d) fused formulation per element. ----
@@ -322,7 +360,7 @@ def main():
     # ---- CPU baseline: the oracle port on the box's host cores, bounded sample of the same workload ----
     if world == 1:
         try:
-            val, dt, cores, nd = time_cpu_port(nx, nb, omega, 3, 1)
+            val, dt, cores, nd, _ = time_cpu_port(nx, nb, omega, 3, 1)
             line["cpu_baseline"] = {"value": val, "unit": UNIT, "cores": cores, "kind": "port",
                                     "sample": "the full uniform_rect(%d) n_basis %d workload, 3 applies of %.2f s (+1 warm-up)" % (nx, nb, dt)}
         except Exception as e:  # the checker is optional for the number, never for the product
