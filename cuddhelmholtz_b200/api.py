@@ -12,6 +12,7 @@ streams here) or raw device addresses (int).
     StiffnessMatrix / MassMatrix / ...         same names; .action(x, y) and .action(c, x, y)
     gmres(n, x, A, b, [P,] m, maxit, tol,..)   gmres(n, x, A, b, m, maxit, tol, P=None, ...)
     DDH(omega, h_a, fem, nx, ny)               DDH(omega, h_a, fem, nx, ny, block=16)
+    (new) DDHTransfer(ddh)                     DDHTransfer(ddh, max_bytes=0): the same operator with T assembled
 """
 import ctypes as C
 import numpy as np
@@ -637,6 +638,72 @@ class DDH:
 
     def _as_apply(self):
         return C.cast(load().cuddh_b200_ddh_as_apply, C.c_void_p), self._h
+
+    def transfer_slots(self):
+        """Host-only slot maps of the assembled operator (DDHTransfer): (inp, out, orphans). inp[p, k] / out[p, k] is the slot that
+        local input / output k of subdomain p reads / writes (-1: face DOF on the physical boundary), shape (n_domains, 2F); k < F is
+        the lambda entry, k >= F the mu entry of face position k mod F (boundary ring of the subdomain grid, ascending Y*n1 + X).
+        orphans: ascending slots that no subdomain writes."""
+        tf = C.c_int()
+        check(load().cuddh_b200_ddh_transfer_slots(self._h, None, None, 0, C.byref(tf)))
+        nd = self.info()["n_domains"]
+        inp = np.zeros((nd, tf.value), np.int32)
+        out = np.zeros((nd, tf.value), np.int32)
+        check(load().cuddh_b200_ddh_transfer_slots(self._h, _vp(inp), _vp(out), inp.size, C.byref(tf)))
+        cnt = C.c_int64()
+        check(load().cuddh_b200_ddh_transfer_orphans(self._h, None, 0, C.byref(cnt)))
+        orphans = np.zeros(cnt.value, np.int32)
+        check(load().cuddh_b200_ddh_transfer_orphans(self._h, _vp(orphans), orphans.size, C.byref(cnt)))
+        return inp, out, orphans
+
+
+class DDHTransfer:
+    """The DDH operator with its trace map T assembled: one dense 2F x 2F FP32 block per subdomain, probed once with 2F WaveHoltz
+    actions, after which action(x, y) = x - T x is one streaming batched matvec. Same linear map as ddh.action (bitwise on unit
+    vectors); rhs / postprocess / array are the DDH's own, so it stands in for the DDH in gmres(...) and DDHPreconditioner.
+    max_bytes: device memory it may take (0 = whatever is free); CuddhError naming the bytes needed if the blocks do not fit."""
+
+    def __init__(self, ddh, max_bytes=0):
+        self.ddh = ddh  # the DDH handle must outlive this one
+        self.fem = ddh.fem
+        self._h = C.c_void_p()
+        check(load().cuddh_b200_ddh_transfer_create(ddh._h, int(max_bytes), _stream(), C.byref(self._h)))
+
+    def __del__(self):
+        _destroy("cuddh_b200_ddh_transfer_destroy", self)
+
+    def size(self):
+        return self.ddh.size()
+
+    def action(self, x, y):
+        check(load().cuddh_b200_ddh_transfer_action(self._h, _ptr(x), _ptr(y), _stream()))
+
+    def rhs(self, f, b):
+        self.ddh.rhs(f, b)
+
+    def postprocess(self, lam, f, u):
+        self.ddh.postprocess(lam, f, u)
+
+    def array(self, name):
+        return self.ddh.array(name)
+
+    def info(self):
+        v = np.zeros(6, np.int64)
+        check(load().cuddh_b200_ddh_transfer_info(self._h, _vp(v)))
+        keys = ["n_domains", "two_f", "block_bytes", "bytes_per_action", "probe_launches"]
+        d = {k: int(x) for k, x in zip(keys, v)}
+        d["probe_ms"] = float(v[5]) / 1000.0
+        return d
+
+    def block(self, dom):
+        """host copy of M_dom, shape (2F, 2F): column k = T's response at the subdomain's outputs to a 1 at its input k"""
+        tf = self.info()["two_f"]
+        out = np.zeros((tf, tf), np.float32)  # C order of the column-major block -> transpose
+        check(load().cuddh_b200_ddh_transfer_get_block(self._h, int(dom), _vp(out)))
+        return out.T.copy()
+
+    def _as_apply(self):
+        return C.cast(load().cuddh_b200_ddh_transfer_as_apply, C.c_void_p), self._h
 
 
 class DDHPreconditioner:

@@ -162,6 +162,14 @@ def _proto(lib):
         "cuddh_b200_ddh_info": (C.c_int, [c_vp, c_vp, P(C.c_double)]),
         "cuddh_b200_ddh_get_array": (C.c_int, [c_vp, C.c_char_p, c_vp, c_i64, P(c_i64)]),
         "cuddh_b200_ddh_flops": (C.c_double, [c_vp]),
+        "cuddh_b200_ddh_transfer_slots": (C.c_int, [c_vp, c_vp, c_vp, c_i64, P(C.c_int)]),
+        "cuddh_b200_ddh_transfer_orphans": (C.c_int, [c_vp, c_vp, c_i64, P(c_i64)]),
+        "cuddh_b200_ddh_transfer_create": (C.c_int, [c_vp, c_i64, c_vp, P(c_vp)]),
+        "cuddh_b200_ddh_transfer_destroy": (C.c_int, [c_vp]),
+        "cuddh_b200_ddh_transfer_action": (C.c_int, [c_vp, c_dp, c_dp, c_vp]),
+        "cuddh_b200_ddh_transfer_as_apply": (C.c_int, [c_vp, c_dp, c_dp, c_vp]),
+        "cuddh_b200_ddh_transfer_info": (C.c_int, [c_vp, c_vp]),
+        "cuddh_b200_ddh_transfer_get_block": (C.c_int, [c_vp, C.c_int, c_vp]),
     }
     for name, (res, args) in sig.items():
         fn = getattr(lib, name)

@@ -60,6 +60,7 @@ struct cuddh_ensemble_s { std::unique_ptr<Ensemble> e; };
 struct cuddh_comm_s { std::unique_ptr<Comm> c; };
 struct cuddh_ddh_dist_s { std::unique_ptr<DdhDist> d; };
 struct cuddh_slab_s { std::unique_ptr<SlabHalo> h; };
+struct cuddh_ddh_transfer_s { std::unique_ptr<DDHTransfer> t; };
 
 static inline cudaStream_t S(void * s) { return (cudaStream_t)s; }
 
@@ -997,6 +998,75 @@ int cuddh_b200_ddh_dist_postprocess(cuddh_ddh_dist_t h, const float * lambda, co
 int cuddh_b200_ddh_dist_as_apply(void * h, const float * x, float * y, void * stream)
 {
     return cuddh_b200_ddh_dist_action((cuddh_ddh_dist_t)h, x, y, stream);
+}
+
+// ---- assembled DDH interface operator ----
+int cuddh_b200_ddh_transfer_slots(cuddh_ddh_t d, int * h_in, int * h_out, int64_t cap, int * two_f)
+{
+    CB_TRY
+    TransferSlots S;
+    transfer_slots(*d->d, S);
+    if (two_f)
+        *two_f = S.two_f;
+    if (h_in || h_out)
+        CB_REQUIRE((int64_t)S.in.size() <= cap, "ddh_transfer_slots: output buffer too small");
+    if (h_in)
+        std::memcpy(h_in, S.in.data(), S.in.size() * sizeof(int));
+    if (h_out)
+        std::memcpy(h_out, S.out.data(), S.out.size() * sizeof(int));
+    CB_CATCH
+}
+int cuddh_b200_ddh_transfer_orphans(cuddh_ddh_t d, int * h_out, int64_t cap, int64_t * count)
+{
+    CB_TRY
+    TransferSlots S;
+    transfer_slots(*d->d, S);
+    if (count)
+        *count = (int64_t)S.orphans.size();
+    if (h_out) {
+        CB_REQUIRE((int64_t)S.orphans.size() <= cap, "ddh_transfer_orphans: output buffer too small");
+        std::memcpy(h_out, S.orphans.data(), S.orphans.size() * sizeof(int));
+    }
+    CB_CATCH
+}
+int cuddh_b200_ddh_transfer_create(cuddh_ddh_t d, int64_t max_bytes, void * stream, cuddh_ddh_transfer_t * out)
+{
+    CB_TRY
+    *out = new cuddh_ddh_transfer_s{std::unique_ptr<DDHTransfer>(new DDHTransfer(d->d.get(), max_bytes, S(stream)))};
+    CB_CATCH
+}
+int cuddh_b200_ddh_transfer_destroy(cuddh_ddh_transfer_t h)
+{
+    delete h;
+    return 0;
+}
+int cuddh_b200_ddh_transfer_action(cuddh_ddh_transfer_t h, const float * x, float * y, void * stream)
+{
+    CB_TRY
+    h->t->action(x, y, S(stream));
+    CB_CATCH
+}
+int cuddh_b200_ddh_transfer_as_apply(void * h, const float * x, float * y, void * stream)
+{
+    return cuddh_b200_ddh_transfer_action((cuddh_ddh_transfer_t)h, x, y, stream);
+}
+int cuddh_b200_ddh_transfer_info(cuddh_ddh_transfer_t h, int64_t * info)
+{
+    CB_TRY
+    const DDHTransfer & T = *h->t;
+    info[0] = T.slots.n_domains;
+    info[1] = T.slots.two_f;
+    info[2] = T.block_bytes();
+    info[3] = T.bytes_per_action();
+    info[4] = T.probe_launches;
+    info[5] = (int64_t)(T.probe_ms * 1000.0 + 0.5);
+    CB_CATCH
+}
+int cuddh_b200_ddh_transfer_get_block(cuddh_ddh_transfer_t h, int dom, float * h_out)
+{
+    CB_TRY
+    h->t->get_block(dom, h_out);
+    CB_CATCH
 }
 
 } // extern "C"

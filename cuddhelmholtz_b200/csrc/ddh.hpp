@@ -80,6 +80,43 @@ namespace cb200
                  const Redirect * redirect = nullptr);
     };
 
+    // Slot maps of the assembled interface operator (DDHTransfer). T = DDH's trace map is block-sparse: subdomain p reads the
+    // (lambda, mu) pairs of its own incoming slots and writes its own outgoing slots, so T is one dense 2F x 2F block per subdomain
+    // (F = mx_fdof face DOFs) between a gather and a scatter. Face position f = 0..F-1 numbers the boundary ring of the n1 x n1
+    // subdomain grid in ascending grid index Y*n1 + X, the same for every subdomain. Local input / output k < F is the lambda
+    // entry of face position k, k >= F the mu entry of face position k - F. Host only.
+    struct TransferSlots
+    {
+        int two_f = 0, n_domains = 0;
+        int64_t n_lambda = 0;
+        std::vector<int> face_at;    // (F) grid index of face position f
+        std::vector<int> in, out;    // (2F, n_domains): slot of the vector that local input / output k of subdomain p reads / writes,
+                                     // -1 = face DOF on the physical boundary (no slot)
+        std::vector<int> orphans;    // ascending slots of [0, 2 n_lambda) that no subdomain writes
+    };
+    // builds the maps from hg_bin / hg_bout; throws unless every slot has at most one reader and at most one writer
+    void transfer_slots(const DDH & D, TransferSlots & S);
+
+    // Assembled DDH operator: y = x - T x with T stored as the probed per-subdomain blocks M_p (2F x 2F, FP32, column-major,
+    // subdomain-contiguous). Creation probes T with 2F actions of the WaveHoltz kernel (input k set to 1 in every subdomain at
+    // once), so every column is that kernel's own output; an action is one streaming batched matvec. `ddh` must outlive this.
+    struct DDHTransfer
+    {
+        DDH * ddh;
+        TransferSlots slots;
+        DevBuf<float> d_M;
+        DevBuf<int> d_in, d_out, d_orphans;
+        int64_t probe_launches = 0;
+        double probe_ms = 0.0;
+
+        // max_bytes: device memory the handle may take (0 = what cudaMemGetInfo reports free); creation is synchronous on s
+        DDHTransfer(DDH * ddh, int64_t max_bytes, cudaStream_t s);
+        int64_t block_bytes() const { return (int64_t)slots.two_f * slots.two_f * slots.n_domains * (int64_t)sizeof(float); }
+        int64_t bytes_per_action() const;   // blocks + maps + gathered inputs + written outputs + orphan copies
+        void action(const float * x, float * y, cudaStream_t s); // y = x - T x; x and y must not overlap
+        void get_block(int dom, float * h_out) const;            // host copy of M_dom (2F x 2F, column-major)
+    };
+
     // contiguous block of subdomains of `rank` (subdomain ids are row-major over the subdomain grid -> row slabs)
     void subdomain_range(int n_domains, int rank, int world, int & begin, int & end);
 

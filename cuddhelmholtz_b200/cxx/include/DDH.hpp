@@ -46,8 +46,35 @@ namespace cuddh
         /// y <- (I - T) x
         void action(const float * x, float * y) const override { cuddh_check(cuddh_b200_ddh_action(h.get(), x, y, nullptr)); }
 
+        /// the library handle (include/cuddh_b200.h)
+        cuddh_ddh_t handle() const { return h.get(); }
+
     private:
         std::shared_ptr<cuddh_ddh_s> h;
+    };
+
+    /// The same operator as DDH with its interface map T assembled: one dense 2F x 2F block per subdomain, probed once with 2F
+    /// WaveHoltz actions; action() is then one streaming batched matvec, y <- (I - T) x. The DDH must outlive this object.
+    class DDHTransfer : public SinglePrecisionOperator
+    {
+    public:
+        /// max_bytes: device memory the blocks may take, 0 = whatever is free (throws with the bytes needed if they do not fit)
+        explicit DDHTransfer(const DDH & ddh, int64_t max_bytes = 0) : ddh(ddh)
+        {
+            cuddh_ddh_transfer_t raw = nullptr;
+            cuddh_check(cuddh_b200_ddh_transfer_create(ddh.handle(), max_bytes, nullptr, &raw));
+            h.reset(raw, [](cuddh_ddh_transfer_t p) { cuddh_b200_ddh_transfer_destroy(p); });
+        }
+
+        int size() const { return ddh.size(); }
+        void rhs(const double * f, float * b) const { ddh.rhs(f, b); }
+        void postprocess(const float * lambda, const double * f, double * u) const { ddh.postprocess(lambda, f, u); }
+        /// y <- (I - T) x  (x and y must not overlap)
+        void action(const float * x, float * y) const override { cuddh_check(cuddh_b200_ddh_transfer_action(h.get(), x, y, nullptr)); }
+
+    private:
+        const DDH & ddh;
+        std::shared_ptr<cuddh_ddh_transfer_s> h;
     };
 } // namespace cuddh
 

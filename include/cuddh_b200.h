@@ -313,6 +313,32 @@ int cuddh_b200_ddh_dist_apply_T(cuddh_ddh_dist_t h, const float * x, float * t, 
 int cuddh_b200_ddh_dist_postprocess(cuddh_ddh_dist_t h, const float * lambda, const double * f, double * u, void * stream);
 int cuddh_b200_ddh_dist_as_apply(void * dist_handle, const float * x, float * y, void * stream); /* cuddh_apply_f_fn */
 
+/* ---- assembled DDH interface operator (new): the same linear map as cuddh_b200_ddh_action, stored -----------------------
+ * T is block-sparse: subdomain p reads only its incoming (lambda, mu) slots and writes only its outgoing ones, so T is one dense
+ * real block M_p of size 2F x 2F per subdomain (F = face DOFs per subdomain, 48 / 56 / 96 / 112 for n_basis 4 / 8 and block 16 /
+ * 32). Face position f numbers the boundary ring of the subdomain's DOF grid in ascending grid index Y*n1 + X (the same order in
+ * every subdomain); local input / output k < F is the lambda entry of face position k, k >= F the mu entry of position k - F.
+ * Creation probes T with 2F WaveHoltz actions (columns are the DDH kernel's own outputs); an action is then one streaming
+ * batched matvec (y = x - T x, deterministic, one launch) instead of 5 x nt time steps per subdomain. Memory: n_domains * 4F^2 * 4
+ * bytes. The cuddh_ddh_t handle must outlive the transfer handle. */
+typedef struct cuddh_ddh_transfer_s * cuddh_ddh_transfer_t;
+/* host only (no GPU needed): slot maps (2F, n_domains) column-major, entry k + 2F p = slot read (h_in) / written (h_out) by
+ * local input / output k of subdomain p, -1 on the physical boundary. cap: capacity of each array in ints; with h_in == h_out ==
+ * NULL only *two_f is returned. Fails unless every slot has at most one reader and at most one writer. */
+int cuddh_b200_ddh_transfer_slots(cuddh_ddh_t d, int * h_in, int * h_out, int64_t cap, int * two_f);
+/* host only: ascending slots of [0, DDH::size()) that no subdomain writes (orphans: y = x there); h_out == NULL -> count only */
+int cuddh_b200_ddh_transfer_orphans(cuddh_ddh_t d, int * h_out, int64_t cap, int64_t * count);
+/* probes the blocks, synchronous on `stream`. max_bytes: device memory the handle may take, 0 = what cudaMemGetInfo reports free;
+ * if blocks + maps + probe vectors do not fit, fails with a message naming the bytes needed */
+int cuddh_b200_ddh_transfer_create(cuddh_ddh_t d, int64_t max_bytes, void * stream, cuddh_ddh_transfer_t * out);
+int cuddh_b200_ddh_transfer_destroy(cuddh_ddh_transfer_t h);
+int cuddh_b200_ddh_transfer_action(cuddh_ddh_transfer_t h, const float * x, float * y, void * stream); /* y = x - T x; no overlap */
+int cuddh_b200_ddh_transfer_as_apply(void * transfer_handle, const float * x, float * y, void * stream); /* cuddh_apply_f_fn */
+/* info[0..5] = n_domains, 2F, block bytes, bytes moved per action, probe launches, probe time in microseconds */
+int cuddh_b200_ddh_transfer_info(cuddh_ddh_transfer_t h, int64_t * info);
+/* host copy of M_dom: (2F, 2F) column-major floats */
+int cuddh_b200_ddh_transfer_get_block(cuddh_ddh_transfer_t h, int dom, float * h_out);
+
 #ifdef __cplusplus
 }
 #endif
