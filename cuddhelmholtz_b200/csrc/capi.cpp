@@ -445,11 +445,8 @@ int64_t cuddh_b200_operator_bytes(cuddh_operator_t op)
 {
     if (op->vol)
         return (int64_t)op->vol->algorithmic_bytes();
-    if (op->helm) {
-        // fused-read formulation of SURVEY §8(d): 24nqS^2 + 8nqM^2 + 4nb^2 + 32(nb-1)^2 per element
-        const int nb = op->helm->fem->nb, qs = op->helm->S->nq, qm = op->helm->M->nq;
-        return (int64_t)op->helm->fem->n_elem * (24ll * qs * qs + 8ll * qm * qm + 4ll * nb * nb + 32ll * (nb - 1) * (nb - 1));
-    }
+    if (op->helm)
+        return (int64_t)op->helm->algorithmic_bytes();
     return 0;
 }
 int64_t cuddh_b200_operator_bytes_moved(cuddh_operator_t op)
@@ -470,10 +467,11 @@ int cuddh_b200_operator_is_affine(cuddh_operator_t op)
 }
 int cuddh_b200_operator_kernel_kind(cuddh_operator_t op)
 {
+    auto kind = [](const VolumeOp & v) { return v.kind == VolumeKernel::ThreadPerElement ? 1 : v.kind == VolumeKernel::ThreadPair ? 3 : 0; };
     if (op->vol)
-        return op->vol->tpe ? 1 : (op->vol->pair ? 3 : 0);
+        return kind(*op->vol);
     if (op->helm)
-        return op->helm->fused ? 2 : (op->helm->S->tpe ? 1 : (op->helm->S->pair ? 3 : 0));
+        return op->helm->fused ? 2 : kind(*op->helm->S);
     return -1;
 }
 

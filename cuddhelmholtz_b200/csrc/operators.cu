@@ -1038,57 +1038,68 @@ namespace cb200
             return v ? atoi(v) : dflt;
         }
 
-        template <int NB, int NQ, bool STIFF>
-        void launch_volume(VolumeOp & op, const PlanDev & pd, const Plan & plan, double c, int accumulate, const double * x,
-                           double * y, cudaStream_t s)
+        PlanDev plan_dev(const Plan & plan)
         {
-            constexpr int EPW = 32 / NQ;
-            constexpr int SCR = scr_layout<NB, NQ, STIFF>().S;
-            const int n_pass = (plan.PE + EPW - 1) / EPW;
-            static const int warps_override = env_int("CUDDH_B200_WARPS", 0);
-            const int nwarps = warps_override > 0 ? std::min(warps_override, 16) : pick_warps(n_pass);
-            size_t smem = sizeof(double) * ((size_t)plan.max_pdof + (size_t)plan.PE * NB * NB + (size_t)nwarps * EPW * SCR) +
-                          sizeof(int) * (size_t)plan.max_pdof + sizeof(uint16_t) * ((size_t)2 * plan.PE * NB * NB + plan.max_pdof + 2);
-            smem = (smem + 15) & ~size_t(15);
-            Tables<NB, NQ, STIFF> tab;
-            std::memset(&tab, 0, sizeof(tab));
-            for (int q = 0; q < NQ; ++q)
-                for (int k = 0; k < NB; ++k) {
-                    tab.Prow[q][k] = op.P[q + NQ * k];
-                    tab.Pcol[k][q] = op.P[q + NQ * k];
-                    if (STIFF) {
-                        tab.Drow[q][k] = op.D[q + NQ * k];
-                        tab.Dcol[k][q] = op.D[q + NQ * k];
-                    }
-                }
-            auto kern = volume_action_kernel<NB, NQ, STIFF>;
-            struct PerDevice
-            {
-                size_t attr_smem = 0;
-                int pf_dist = -1;
-            };
-            static PerDevice per_device[MAX_DEVICES];
+            return PlanDev{plan.d_hdr.p, plan.d_gid.p, plan.d_slot.p, plan.d_L.p, plan.d_cptr.p, plan.d_cent.p, plan.PE, plan.d_Ig.p,
+                           reinterpret_cast<const uint2 *>(plan.d_cent4.p), plan.d_target.p};
+        }
+
+        // launch configuration of `grid` CTAs of 256 threads in clusters of `cluster` along x (attr must outlive it)
+        cudaLaunchConfig_t cluster_config(int grid, size_t smem, int cluster, cudaLaunchAttribute & attr, cudaStream_t s = 0)
+        {
+            cudaLaunchConfig_t cfg = {};
+            cfg.gridDim = dim3((unsigned)grid);
+            cfg.blockDim = dim3(256);
+            cfg.dynamicSmemBytes = smem;
+            cfg.stream = s;
+            attr.id = cudaLaunchAttributeClusterDimension;
+            attr.val.clusterDim.x = (unsigned)cluster;
+            attr.val.clusterDim.y = 1;
+            attr.val.clusterDim.z = 1;
+            cfg.attrs = &attr;
+            cfg.numAttrs = 1;
+            return cfg;
+        }
+
+        // what one kernel instance has been set up for on one device (function attributes are per device)
+        struct DeviceSetup
+        {
+            size_t smem = 0; // dynamic shared-memory limit set so far
+            int wave = 0;    // one wave of resident CTAs: resident CTAs per SM x SM count
+        };
+
+        // Raises the instance's dynamic shared-memory limit whenever a launch needs more than before and asks for the largest
+        // carve-out (several CTAs per SM are needed to overlap the staging / assembly phases of one patch with the contractions
+        // of another). Sizes the wave at the first launch on the device; cluster > 1: the kernel runs as clusters of that many
+        // CTAs, and the wave is clamped to the co-resident clusters.
+        template <class Kern>
+        const DeviceSetup & setup_kernel(DeviceSetup (&per_device)[MAX_DEVICES], Kern kern, int threads, size_t smem, int cluster = 1)
+        {
             int dev = 0;
             cudaGetDevice(&dev);
             CB_REQUIRE(dev >= 0 && dev < MAX_DEVICES, "device ordinal out of range");
-            PerDevice & pdv = per_device[dev];
-            if (smem > pdv.attr_smem) {
+            DeviceSetup & st = per_device[dev];
+            if (smem > st.smem) {
                 CB_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)std::max(smem, (size_t)49152)));
-                // several CTAs per SM are needed to overlap the staging / assembly phases of one patch with the
-                // contractions of another: ask for the largest shared-memory carve-out
                 CB_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared));
-                pdv.attr_smem = std::max(smem, (size_t)49152);
+                st.smem = std::max(smem, (size_t)49152);
             }
-            if (pdv.pf_dist < 0) { // one scheduling wave = resident CTAs per SM x SM count
+            if (!st.wave) {
                 int sms = 148, occ = 1;
                 cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
-                cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, kern, nwarps * 32, smem);
-                pdv.pf_dist = env_int("CUDDH_B200_PFDIST", std::max(occ, 1) * sms);
+                CB_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, kern, threads, smem));
+                st.wave = std::max(1, occ) * sms;
+                if (cluster > 1) {
+                    cudaLaunchAttribute at;
+                    const cudaLaunchConfig_t cfg = cluster_config(st.wave, smem, cluster, at);
+                    int ncl = 0;
+                    if (cudaOccupancyMaxActiveClusters(&ncl, kern, &cfg) == cudaSuccess && ncl > 0)
+                        st.wave = std::min(st.wave, cluster * ncl);
+                    else
+                        cudaGetLastError();
+                }
             }
-            const int pf_dist = pdv.pf_dist;
-            kern<<<(unsigned)plan.n_patches, nwarps * 32, smem, s>>>(tab, pd, op.d_G.p, x, y, op.d_partial.p, c, accumulate,
-                                                                       plan.max_pdof, (int)plan.n_patches, pf_dist);
-            CB_LAUNCHED();
+            return st;
         }
 
         template <int NB, int NQ, bool STIFF>
@@ -1112,9 +1123,39 @@ namespace cb200
                 }
         }
 
-        template <int NB, int NQ, bool STIFF, int NQ2, int RING = 0, bool AFFINE = false>
-        void launch_ws(const VolumeOp & op, const VolumeOp * op2, const PlanDev & pd, const Plan & plan, const WsArgs & args, cudaStream_t s)
+        using LaunchFn = decltype(VolumeOp::launch);
+        using FusedFn = decltype(HelmholtzOp::fused);
+
+        template <int NB, int NQ, bool STIFF>
+        void launch_volume(const VolumeOp & op, double c, int accumulate, const double * x, double * y, cudaStream_t s)
         {
+            constexpr int EPW = 32 / NQ;
+            constexpr int SCR = scr_layout<NB, NQ, STIFF>().S;
+            const Plan & plan = *op.plan;
+            const int n_pass = (plan.PE + EPW - 1) / EPW;
+            static const int warps_override = env_int("CUDDH_B200_WARPS", 0);
+            const int nwarps = warps_override > 0 ? std::min(warps_override, 16) : pick_warps(n_pass);
+            size_t smem = sizeof(double) * ((size_t)plan.max_pdof + (size_t)plan.PE * NB * NB + (size_t)nwarps * EPW * SCR) +
+                          sizeof(int) * (size_t)plan.max_pdof + sizeof(uint16_t) * ((size_t)2 * plan.PE * NB * NB + plan.max_pdof + 2);
+            smem = (smem + 15) & ~size_t(15);
+            Tables<NB, NQ, STIFF> tab;
+            fill_tables(tab, op); // the weighted / scaled rows are not read by this kernel
+            auto kern = volume_action_kernel<NB, NQ, STIFF>;
+            static DeviceSetup per_device[MAX_DEVICES];
+            const DeviceSetup & st = setup_kernel(per_device, kern, nwarps * 32, smem);
+            // L2 prefetch distance in patches: one scheduling wave unless CUDDH_B200_PFDIST is set
+            static const bool pf_set = getenv("CUDDH_B200_PFDIST") != nullptr;
+            static const int pf_env = env_int("CUDDH_B200_PFDIST", 0);
+            const int pf_dist = pf_set ? pf_env : st.wave;
+            kern<<<(unsigned)plan.n_patches, nwarps * 32, smem, s>>>(tab, plan_dev(plan), op.d_G.p, x, y, op.d_partial.p, c, accumulate,
+                                                                       plan.max_pdof, (int)plan.n_patches, pf_dist);
+            CB_LAUNCHED();
+        }
+
+        template <int NB, int NQ, bool STIFF, int NQ2, int RING = 0, bool AFFINE = false>
+        void launch_ws(const VolumeOp & op, const VolumeOp * op2, WsArgs args, cudaStream_t s)
+        {
+            const Plan & plan = *op.plan;
             CB_REQUIRE(plan.PE == 128, "warp-specialised kernel: patches must hold 128 elements");
             constexpr int NI = (NB > 2 ? NB - 2 : 0) * (NB > 2 ? NB - 2 : 0);
             constexpr int NPRa = TpeCfg<NB, NQ, STIFF>::KR / 2, NPRb = NQ2 > 0 ? TpeCfg<NB, (NQ2 > 0 ? NQ2 : 1), false>::KR / 2 : 0;
@@ -1131,56 +1172,17 @@ namespace cb200
             if constexpr (NQ2 > 0)
                 fill_tables(tab2, *op2, args.msc);
             auto kern = volume_action_ws<NB, NQ, STIFF, NQ2, RING, AFFINE>;
-            // one wave of resident CTAs, cached per device (function attributes are per device too)
-            static int grid_of_device[MAX_DEVICES] = {};
-            int dev = 0;
-            cudaGetDevice(&dev);
-            CB_REQUIRE(dev >= 0 && dev < MAX_DEVICES, "device ordinal out of range");
-            int & grid = grid_of_device[dev];
-            if (!grid) {
-                CB_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)std::max(smem, (size_t)49152)));
-                CB_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared));
-                int sms = 148, occ = 1;
-                cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
-                CB_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, kern, 256, smem));
-                int gsz = std::max(1, occ) * sms;
-                if (NQ2 > 0) { // launched as clusters of two CTAs: ask how many of those are co-resident
-                    cudaLaunchConfig_t cfg = {};
-                    cfg.gridDim = dim3((unsigned)gsz);
-                    cfg.blockDim = dim3(256);
-                    cfg.dynamicSmemBytes = smem;
-                    cudaLaunchAttribute at[1];
-                    at[0].id = cudaLaunchAttributeClusterDimension;
-                    at[0].val.clusterDim.x = 2;
-                    at[0].val.clusterDim.y = 1;
-                    at[0].val.clusterDim.z = 1;
-                    cfg.attrs = at;
-                    cfg.numAttrs = 1;
-                    int ncl = 0;
-                    if (cudaOccupancyMaxActiveClusters(&ncl, kern, &cfg) == cudaSuccess && ncl > 0)
-                        gsz = std::min(gsz, 2 * ncl);
-                    else
-                        cudaGetLastError();
-                }
-                grid = gsz;
-            }
+            static DeviceSetup per_device[MAX_DEVICES];
+            const int grid = setup_kernel(per_device, kern, 256, smem, NQ2 > 0 ? 2 : 1).wave;
             const int nf = std::max(args.n_fields, 1);
             const int cap = max_persistent_ctas(); // test / tuning knob: fewer CTAs = more patches per persistent CTA
             const int wave = cap > 0 ? std::max(nf, std::min(grid, cap)) : grid;
             const int g = (int)std::min<int64_t>(wave / nf, plan.n_patches) * nf;
+            const PlanDev pd = plan_dev(plan);
+            args.n_patches = (int)plan.n_patches;
             if (nf > 1) { // one cluster = the CTAs that walk the same patches, one field each
-                cudaLaunchConfig_t cfg = {};
-                cfg.gridDim = dim3((unsigned)g);
-                cfg.blockDim = dim3(256);
-                cfg.dynamicSmemBytes = smem;
-                cfg.stream = s;
-                cudaLaunchAttribute at[1];
-                at[0].id = cudaLaunchAttributeClusterDimension;
-                at[0].val.clusterDim.x = (unsigned)nf;
-                at[0].val.clusterDim.y = 1;
-                at[0].val.clusterDim.z = 1;
-                cfg.attrs = at;
-                cfg.numAttrs = 1;
+                cudaLaunchAttribute at;
+                const cudaLaunchConfig_t cfg = cluster_config(g, smem, nf, at, s);
                 CB_CUDA(cudaLaunchKernelEx(&cfg, kern, tab, tab2, pd, args));
             }
             else
@@ -1189,8 +1191,7 @@ namespace cb200
         }
 
         template <int NB, int NQ, bool STIFF, int RING = 0, bool AFFINE = false>
-        void launch_volume_ws(VolumeOp & op, const PlanDev & pd, const Plan & plan, double c, int accumulate, const double * x,
-                              double * y, cudaStream_t s)
+        void launch_volume_ws(const VolumeOp & op, double c, int accumulate, const double * x, double * y, cudaStream_t s)
         {
             WsArgs a{};
             a.G1 = reinterpret_cast<const double2 *>(op.d_G.p);
@@ -1202,9 +1203,8 @@ namespace cb200
             a.c[0] = a.c[1] = c;
             a.msc = 1.0;
             a.accumulate = accumulate;
-            a.n_patches = (int)plan.n_patches;
             a.n_fields = 1;
-            launch_ws<NB, NQ, STIFF, 0, RING, AFFINE>(op, nullptr, pd, plan, a, s);
+            launch_ws<NB, NQ, STIFF, 0, RING, AFFINE>(op, nullptr, a, s);
         }
 
         // thread-pair-per-element kernel (volume_pair.cuh): n_basis 6-9
@@ -1241,8 +1241,9 @@ namespace cb200
 
         // one launch of the thread-pair kernel: a single operator (NQ2 == 0, op2 == nullptr) or the fused S + msc * M of one field
         template <int NB, int NQ, bool STIFF, bool AFFINE, int NQ2>
-        void launch_pair(const VolumeOp & op, const VolumeOp * op2, const PlanDev & pd, const Plan & plan, PairArgs a, cudaStream_t s)
+        void launch_pair(const VolumeOp & op, const VolumeOp * op2, PairArgs a, cudaStream_t s)
         {
+            const Plan & plan = *op.plan;
             CB_REQUIRE(plan.PE == 64 && plan.interior_affine, "thread-pair kernel: needs 64-element patches and affine element-interior ids");
             constexpr int NI = 2;
             constexpr int RD = pair_ring_depth<NB, NQ, STIFF, AFFINE>();
@@ -1258,31 +1259,19 @@ namespace cb200
             if constexpr (NQ2 > 0)
                 fill_pair_tables(tab2, *op2, a.msc);
             auto kern = volume_action_pair<NB, NQ, STIFF, AFFINE, RD, NQ2, RD2>;
-            static int grid_of_device[MAX_DEVICES] = {};
-            int dev = 0;
-            cudaGetDevice(&dev);
-            CB_REQUIRE(dev >= 0 && dev < MAX_DEVICES, "device ordinal out of range");
-            int & grid = grid_of_device[dev];
-            if (!grid) {
-                CB_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)std::max(smem, (size_t)49152)));
-                CB_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared));
-                int sms = 148, occ = 1;
-                cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
-                CB_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, kern, 256, smem));
-                grid = std::max(1, occ) * sms;
-            }
+            static DeviceSetup per_device[MAX_DEVICES];
+            const int grid = setup_kernel(per_device, kern, 256, smem).wave;
             a.n_patches = (int)plan.n_patches;
             a.zero = 0;
             const int cap = max_persistent_ctas();
             const int wave = cap > 0 ? std::min(grid, cap) : grid;
             const int g = (int)std::min<int64_t>(wave, plan.n_patches);
-            kern<<<g, 256, smem, s>>>(tab, tab2, pd, a);
+            kern<<<g, 256, smem, s>>>(tab, tab2, plan_dev(plan), a);
             CB_LAUNCHED();
         }
 
         template <int NB, int NQ, bool STIFF, bool AFFINE = false>
-        void launch_volume_pair(VolumeOp & op, const PlanDev & pd, const Plan & plan, double c, int accumulate, const double * x, double * y,
-                                cudaStream_t s)
+        void launch_volume_pair(const VolumeOp & op, double c, int accumulate, const double * x, double * y, cudaStream_t s)
         {
             PairArgs a{};
             a.G = reinterpret_cast<const double2 *>(op.d_G.p);
@@ -1294,24 +1283,103 @@ namespace cb200
             a.c = c;
             a.msc = 1.0;
             a.accumulate = accumulate;
-            launch_pair<NB, NQ, STIFF, AFFINE, 0>(op, nullptr, pd, plan, a, s);
+            launch_pair<NB, NQ, STIFF, AFFINE, 0>(op, nullptr, a, s);
         }
 
-        // fused S + msc * M of one field (Helmholtz composite at n_basis 6-8): stiffness rule nq = nb + 1, weighted-mass rule 1 + 3nb/2 + 1
-        using FusedPairFn = void (*)(const VolumeOp &, const VolumeOp *, const PlanDev &, const Plan &, PairArgs, cudaStream_t);
-        FusedPairFn find_fused_pair_instance(int nb, int nqs, int nqm, bool affine)
+        // stride of the two fields in HelmholtzOp::d_partial2
+        int64_t partial_stride(const HelmholtzOp & h) { return std::max<int64_t>(h.S->plan->n_slots_total, 1); }
+
+        // the volume phase of the fused Helmholtz apply, both fields in one launch (the two CTAs of a cluster); the sign of the
+        // second block row is applied on write
+        template <int NB, int NQS, int NQM, int RING, bool AFFINE>
+        void launch_fused_ws(const HelmholtzOp & h, const double * x, double * y, cudaStream_t s)
         {
-            if (!affine) // stored-metric meshes keep the per-operator launches (see volume_action_pair)
-                return nullptr;
-#define CB_CASE(NB_, NQS_, NQM_)                                                                                       \
-    if (nb == NB_ && nqs == NQS_ && nqm == NQM_)                                                                       \
-        return &launch_pair<NB_, NQS_, true, true, NQM_>;
-            CB_CASE(6, 7, 11) CB_CASE(7, 8, 12) CB_CASE(8, 9, 14) CB_CASE(9, 10, 15)
-#undef CB_CASE
-            return nullptr;
+            WsArgs a{};
+            a.G1 = reinterpret_cast<const double2 *>(h.S->d_G.p);
+            a.G2 = reinterpret_cast<const double2 *>(h.M->d_G.p);
+            a.Gc = h.S->d_Gc.p;
+            a.x = x;
+            a.y = y;
+            a.partial = h.d_partial2.p;
+            a.x_stride = a.y_stride = h.fem->ndof;
+            a.partial_stride = partial_stride(h);
+            a.c[0] = 1.0;
+            a.c[1] = -1.0;
+            a.msc = -h.omega * h.omega;
+            a.accumulate = 0;
+            a.n_fields = 2;
+            launch_ws<NB, NQS, true, NQM, RING, AFFINE>(*h.S, h.M.get(), a, s);
         }
 
-        using LaunchFn = void (*)(VolumeOp &, const PlanDev &, const Plan &, double, int, const double *, double *, cudaStream_t);
+        // the shared-DOF pass of the fused apply, both fields in one launch
+        void assemble_shared_fields(const HelmholtzOp & h, double * y, cudaStream_t s)
+        {
+            const Plan & plan = *h.S->plan;
+            if (plan.n_shared > 0) {
+                assemble_shared_fields_kernel<<<dim3(blocks_for(plan.n_shared, 256), 2), 256, 0, s>>>(
+                    plan.n_shared, plan.d_sh_gid.p, plan.d_sh_ptr.p, h.d_partial2.p, partial_stride(h), y, h.fem->ndof, 1.0, -1.0);
+                CB_LAUNCHED();
+            }
+        }
+
+        // n_basis 6-9: the thread-pair kernel runs S - omega^2 M of one field per launch
+        template <int NB, int NQS, int NQM>
+        void launch_fused_pair(const HelmholtzOp & h, const double * x, double * y, cudaStream_t s)
+        {
+            const int64_t n = h.fem->ndof;
+            for (int f = 0; f < 2; ++f) {
+                PairArgs a{};
+                a.G = reinterpret_cast<const double2 *>(h.S->d_G.p);
+                a.G2 = reinterpret_cast<const double2 *>(h.M->d_G.p);
+                a.Gc = h.S->d_Gc.p;
+                a.x = x + f * n;
+                a.y = y + f * n;
+                a.partial = h.d_partial2.p + f * partial_stride(h);
+                a.c = f == 0 ? 1.0 : -1.0;
+                a.msc = -h.omega * h.omega;
+                a.accumulate = 0;
+                launch_pair<NB, NQS, true, true, NQM>(*h.S, h.M.get(), a, s);
+            }
+        }
+
+        // ------------------------------------------------------------------------------------------
+        // kernel selection
+        // ------------------------------------------------------------------------------------------
+        // The metric-ring variants of one instance family: ring knob value -> instance. A value that is not listed gets the
+        // first entry.
+        template <class Fn>
+        struct RingVariant
+        {
+            int ring;
+            Fn fn;
+        };
+        template <class Fn, size_t N>
+        Fn ring_variant(const RingVariant<Fn> (&family)[N], int ring)
+        {
+            for (const RingVariant<Fn> & v : family)
+                if (v.ring == ring)
+                    return v.fn;
+            return family[0].fn;
+        }
+
+        // stand-alone thread-per-element operators and stored-metric fused ones: 0 = metric rows through registers, 2 / 5 =
+        // shared-memory TMA ring of that many chunks (contract_phase_ring), -5 = per-thread cp.async ring (no row barrier)
+        template <int NB, int NQ, bool STIFF>
+        const RingVariant<LaunchFn> tpe_rings[4] = {{0, &launch_volume_ws<NB, NQ, STIFF, 0>},
+                                                    {-5, &launch_volume_ws<NB, NQ, STIFF, -5>},
+                                                    {2, &launch_volume_ws<NB, NQ, STIFF, 2>},
+                                                    {5, &launch_volume_ws<NB, NQ, STIFF, 5>}};
+        template <int NB, int NQS, int NQM>
+        const RingVariant<FusedFn> fused_stored_rings[4] = {{0, &launch_fused_ws<NB, NQS, NQM, 0, false>},
+                                                            {-5, &launch_fused_ws<NB, NQS, NQM, -5, false>},
+                                                            {2, &launch_fused_ws<NB, NQS, NQM, 2, false>},
+                                                            {5, &launch_fused_ws<NB, NQS, NQM, 5, false>}};
+        // fused affine operators (the ring carries the mass rows): 0 = straight from global memory into registers, 5 = the TMA
+        // ring; any other value: the per-thread cp.async ring of -TR rows
+        template <int NB, int NQS, int NQM, int TR>
+        const RingVariant<FusedFn> fused_affine_rings[3] = {{TR, &launch_fused_ws<NB, NQS, NQM, TR, true>},
+                                                            {0, &launch_fused_ws<NB, NQS, NQM, 0, true>},
+                                                            {5, &launch_fused_ws<NB, NQS, NQM, 5, true>}};
 
         template <bool STIFF>
         LaunchFn find_pair_instance(int nb, int nq, bool affine = false)
@@ -1348,48 +1416,22 @@ namespace cb200
             return nullptr;
         }
 
+        // ring5 / ring4: metric ring of the n_basis 5 / 4 instances of the default rules (stiffness nq = nb + 1, weighted mass)
         template <bool STIFF>
-        LaunchFn find_tpe_instance(int nb, int nq)
+        LaunchFn find_tpe_instance(int nb, int nq, int ring5, int ring4)
         {
 #define CB_CASE(NB_, NQ_)                                                                                              \
     if (nb == NB_ && nq == NQ_)                                                                                        \
         return &launch_volume_ws<NB_, NQ_, STIFF>;
-            // n_basis 5: metric data through the shared-memory ring (see contract_phase_ring)
-            static const int ring = env_int("CUDDH_B200_RING1", 5);
-            if constexpr (STIFF) {
-                if (ring == -5 && nb == 5 && nq == 6) // negative: per-thread cp.async ring (no row barrier)
-                    return &launch_volume_ws<5, 6, true, -5>;
-                if (ring == 2 && nb == 5 && nq == 6)
-                    return &launch_volume_ws<5, 6, true, 2>;
-                if (ring == 5 && nb == 5 && nq == 6)
-                    return &launch_volume_ws<5, 6, true, 5>;
-                static const int ring4 = env_int("CUDDH_B200_RING4", 5);
-                if (ring4 == -5 && nb == 4 && nq == 5)
-                    return &launch_volume_ws<4, 5, true, -5>;
-                if (ring4 == 2 && nb == 4 && nq == 5)
-                    return &launch_volume_ws<4, 5, true, 2>;
-                if (ring4 == 5 && nb == 4 && nq == 5)
-                    return &launch_volume_ws<4, 5, true, 5>;
-            }
-            else {
-                if (ring == -5 && nb == 5 && nq == 9)
-                    return &launch_volume_ws<5, 9, false, -5>;
-                if (ring == 2 && nb == 5 && nq == 9)
-                    return &launch_volume_ws<5, 9, false, 2>;
-                if (ring == 5 && nb == 5 && nq == 9)
-                    return &launch_volume_ws<5, 9, false, 5>;
-                static const int ring4 = env_int("CUDDH_B200_RING4", 5);
-                if (ring4 == -5 && nb == 4 && nq == 8)
-                    return &launch_volume_ws<4, 8, false, -5>;
-                if (ring4 == 2 && nb == 4 && nq == 8)
-                    return &launch_volume_ws<4, 8, false, 2>;
-                if (ring4 == 5 && nb == 4 && nq == 8)
-                    return &launch_volume_ws<4, 8, false, 5>;
-            }
+            constexpr int NQ5 = STIFF ? 6 : 9, NQ4 = STIFF ? 5 : 8;
+            if (nb == 5 && nq == NQ5)
+                return ring_variant(tpe_rings<5, NQ5, STIFF>, ring5);
+            if (nb == 4 && nq == NQ4)
+                return ring_variant(tpe_rings<4, NQ4, STIFF>, ring4);
             CB_CASE(2, 3) CB_CASE(3, 4) CB_CASE(4, 5) CB_CASE(5, 6)
             CB_CASE(3, 5) CB_CASE(4, 6) CB_CASE(5, 7)
             if constexpr (!STIFF) {
-                CB_CASE(2, 5) CB_CASE(3, 6) CB_CASE(4, 8) CB_CASE(5, 9)
+                CB_CASE(2, 5) CB_CASE(3, 6)
             }
 #undef CB_CASE
             return nullptr;
@@ -1411,44 +1453,73 @@ namespace cb200
 #undef CB_CASE
             return nullptr;
         }
-        using FusedFn = void (*)(const VolumeOp &, const VolumeOp *, const PlanDev &, const Plan &, const WsArgs &, cudaStream_t);
-        FusedFn find_fused_instance(int nb, int nqs, int nqm, bool affine = false)
+
+        struct VolumeChoice
         {
-            if (affine) {
-                // mass rows through the shared-memory ring (5) or straight from global memory into registers (0)
-                static const int aring = env_int("CUDDH_B200_AFFINE_RING", -5);
-                // (negative: per-thread cp.async ring of that many rows)
-                if (nb == 5 && nqs == 6 && nqm == 9)
-                    return aring == 0 ? &launch_ws<5, 6, true, 9, 0, true> : aring == 5 ? &launch_ws<5, 6, true, 9, 5, true>
-                         : &launch_ws<5, 6, true, 9, -5, true>;
-                if (nb == 4 && nqs == 5 && nqm == 8)
-                    return aring == 0 ? &launch_ws<4, 5, true, 8, 0, true> : aring == 5 ? &launch_ws<4, 5, true, 8, 5, true>
-                         : &launch_ws<4, 5, true, 8, -4, true>;
-                return nullptr;
+            VolumeKernel kind;
+            bool affine;     // stiffness from per-element metric constants (every element a parallelogram)
+            LaunchFn launch; // null for Generic
+            Plan * plan;
+        };
+
+        // Which kernel runs a stiffness / mass operator. The only reader of the knobs that select one: CUDDH_B200_FORCE_GENERIC,
+        // CUDDH_B200_TPE, CUDDH_B200_PAIR, CUDDH_B200_AFFINE (0 = stored metric), CUDDH_B200_RING1 / RING4 (metric ring of the
+        // n_basis 5 / 4 thread-per-element operators).
+        VolumeChoice select_volume_kernel(H1Space * fem, int nb, int nq, bool stiff, bool want_affine)
+        {
+            const LaunchFn lane = stiff ? find_instance<true>(nb, nq) : find_instance<false>(nb, nq);
+            if (getenv("CUDDH_B200_FORCE_GENERIC") != nullptr || !lane)
+                return {VolumeKernel::Generic, false, nullptr, &fem->get_plan()};
+            auto affine_ok = [&] { return want_affine && stiff && env_int("CUDDH_B200_AFFINE", 1) != 0 && fem->all_affine(); };
+            if (env_int("CUDDH_B200_TPE", 1) != 0) {
+                const int ring5 = env_int("CUDDH_B200_RING1", 5), ring4 = env_int("CUDDH_B200_RING4", 5);
+                const LaunchFn tpe = stiff ? find_tpe_instance<true>(nb, nq, ring5, ring4) : find_tpe_instance<false>(nb, nq, ring5, ring4);
+                if (tpe) {
+                    const LaunchFn aff = stiff ? find_affine_instance(nb, nq) : nullptr;
+                    const bool affine = aff && affine_ok();
+                    return {VolumeKernel::ThreadPerElement, affine, affine ? aff : tpe, &fem->get_plan_tpe()};
+                }
             }
-            // stored-metric fused instances: per-thread chunk ring (n_basis 5: 0.704 ms against 0.719 ms of the TMA ring, n_basis 4: 0.388 / 0.437)
-            static const int ring = env_int("CUDDH_B200_RING", -5);
-#define CB_CASE(NB_, NQS_, NQM_)                                                                                       \
-    if (nb == NB_ && nqs == NQS_ && nqm == NQM_)                                                                       \
-        return &launch_ws<NB_, NQS_, true, NQM_>;
-            // shared-memory metric ring for the register-bound n_basis 5 instance
-            if (nb == 5 && nqs == 6 && nqm == 9 && ring == -5)
-                return &launch_ws<5, 6, true, 9, -5>;
-            if (nb == 5 && nqs == 6 && nqm == 9 && ring == 2)
-                return &launch_ws<5, 6, true, 9, 2>;
-            if (nb == 5 && nqs == 6 && nqm == 9 && ring == 5)
-                return &launch_ws<5, 6, true, 9, 5>;
-            // n_basis 4: per-thread chunk ring (measured 0.437 -> 0.388 ms; at n_basis 5 the two rings tie, 0.720 / 0.717 ms)
-            static const int ring4 = env_int("CUDDH_B200_RING4F", -5);
-            if (nb == 4 && nqs == 5 && nqm == 8 && ring4 == -5)
-                return &launch_ws<4, 5, true, 8, -5>;
-            if (nb == 4 && nqs == 5 && nqm == 8 && ring4 == 2)
-                return &launch_ws<4, 5, true, 8, 2>;
-            if (nb == 4 && nqs == 5 && nqm == 8 && ring4 == 5)
-                return &launch_ws<4, 5, true, 8, 5>;
+            if (env_int("CUDDH_B200_PAIR", 1) != 0) {
+                const bool affine = nb >= 6 && affine_ok();
+                const LaunchFn pair = stiff ? find_pair_instance<true>(nb, nq, affine) : find_pair_instance<false>(nb, nq);
+                // never with H1Space's own numbering and the default patch shape (the CUDDH_B200_TPE_PX / PY experiment knobs can
+                // change the latter): the lane-per-row kernel serves such a plan
+                if (pair) {
+                    Plan & plan = fem->get_plan_tpe();
+                    if (plan.PE == 64 && plan.interior_affine)
+                        return {VolumeKernel::ThreadPair, affine, pair, &plan};
+                }
+            }
+            return {VolumeKernel::LanePerRow, false, lane, &fem->get_plan()};
+        }
+
+        // The fused volume phase of the Helmholtz composite, or null when S and M run one by one. The only reader of the knobs
+        // of the fused kernels: CUDDH_B200_FUSED, CUDDH_B200_AFFINE_RING, CUDDH_B200_RING (n_basis 5) / RING4F (n_basis 4).
+        FusedFn select_fused_kernel(const VolumeOp & S, const VolumeOp & M)
+        {
+            if (S.kind != M.kind || S.plan != M.plan || env_int("CUDDH_B200_FUSED", 1) == 0)
+                return nullptr;
             // default stiffness rule nq = nb + 1 with the weighted-mass rule nq = 1 + 3nb/2 + 1 (examples/Helmholtz.hpp)
-            CB_CASE(2, 3, 5) CB_CASE(3, 4, 6) CB_CASE(4, 5, 8) CB_CASE(5, 6, 9)
-#undef CB_CASE
+            auto rule = [&](int nb, int nqs, int nqm) { return S.nb == nb && S.nq == nqs && M.nq == nqm; };
+            if (S.kind == VolumeKernel::ThreadPerElement && S.affine) {
+                const int ring = env_int("CUDDH_B200_AFFINE_RING", -5);
+                if (rule(5, 6, 9)) return ring_variant(fused_affine_rings<5, 6, 9, -5>, ring);
+                if (rule(4, 5, 8)) return ring_variant(fused_affine_rings<4, 5, 8, -4>, ring);
+            }
+            else if (S.kind == VolumeKernel::ThreadPerElement) {
+                // stored metric: per-thread chunk ring (n_basis 5: 0.704 ms against 0.719 ms of the TMA ring, n_basis 4: 0.388 / 0.437)
+                if (rule(5, 6, 9)) return ring_variant(fused_stored_rings<5, 6, 9>, env_int("CUDDH_B200_RING", -5));
+                if (rule(4, 5, 8)) return ring_variant(fused_stored_rings<4, 5, 8>, env_int("CUDDH_B200_RING4F", -5));
+                if (rule(2, 3, 5)) return &launch_fused_ws<2, 3, 5, 0, false>;
+                if (rule(3, 4, 6)) return &launch_fused_ws<3, 4, 6, 0, false>;
+            }
+            else if (S.kind == VolumeKernel::ThreadPair && S.affine) { // stored-metric meshes keep the per-operator launches (see volume_action_pair)
+                if (rule(6, 7, 11)) return &launch_fused_pair<6, 7, 11>;
+                if (rule(7, 8, 12)) return &launch_fused_pair<7, 8, 12>;
+                if (rule(8, 9, 14)) return &launch_fused_pair<8, 9, 14>;
+                if (rule(9, 10, 15)) return &launch_fused_pair<9, 10, 15>;
+            }
             return nullptr;
         }
     } // namespace
@@ -1459,18 +1530,10 @@ namespace cb200
     void VolumeOp::apply(double c, int accumulate, const double * x, double * y, cudaStream_t s, int phases)
     {
         NvtxRange nvtx_(stiff ? "cuddh::StiffnessMatrix::action" : "cuddh::MassMatrix::action");
-        Plan & plan = *this->plan;
-        PlanDev pd{plan.d_hdr.p, plan.d_gid.p, plan.d_slot.p, plan.d_L.p, plan.d_cptr.p, plan.d_cent.p, plan.PE, plan.d_Ig.p, reinterpret_cast<const uint2 *>(plan.d_cent4.p), plan.d_target.p};
-        LaunchFn fn = generic ? nullptr : (stiff ? find_instance<true>(nb, nq) : find_instance<false>(nb, nq));
-        if (tpe)
-            fn = affine ? find_affine_instance(nb, nq) : (stiff ? find_tpe_instance<true>(nb, nq) : find_tpe_instance<false>(nb, nq));
-        if (pair)
-            fn = stiff ? find_pair_instance<true>(nb, nq, affine) : find_pair_instance<false>(nb, nq);
-        if (!(phases & 1)) {
-        }
-        else if (fn)
-            fn(*this, pd, plan, c, accumulate, x, y, s);
-        else {
+        const Plan & plan = *this->plan;
+        if ((phases & 1) && launch)
+            launch(*this, c, accumulate, x, y, s);
+        else if (phases & 1) {
             const int nwarps = std::min(8, plan.PE);
             const int SCR = (stiff ? 2 : 1) * nq * nb;
             size_t smem = sizeof(double) * ((size_t)plan.max_pdof + (size_t)plan.PE * nb * nb + (size_t)nwarps * SCR) +
@@ -1478,8 +1541,8 @@ namespace cb200
             smem = (smem + 15) & ~size_t(15);
             CB_REQUIRE(smem <= 227 * 1024, "operator action: patch does not fit in shared memory for this (n_basis, n_quad)");
             CB_CUDA(cudaFuncSetAttribute(volume_action_generic, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)std::max(smem, (size_t)49152)));
-            volume_action_generic<<<(unsigned)plan.n_patches, nwarps * 32, smem, s>>>(nb, nq, stiff ? 1 : 0, d_P.p, d_D.p, pd, d_G.p, x, y,
-                                                                                      d_partial.p, c, accumulate, plan.max_pdof);
+            volume_action_generic<<<(unsigned)plan.n_patches, nwarps * 32, smem, s>>>(nb, nq, stiff ? 1 : 0, d_P.p, d_D.p, plan_dev(plan), d_G.p, x,
+                                                                                      y, d_partial.p, c, accumulate, plan.max_pdof);
             CB_LAUNCHED();
         }
         if (plan.n_shared > 0 && (phases & 2)) {
@@ -1506,7 +1569,15 @@ namespace cb200
 
     namespace
     {
-        void init_volume_common(VolumeOp & op, H1Space * fem, int nq, bool stiff, bool force_generic, bool want_affine = false)
+        // layout of the metric data for the setup kernels (metric_index / metric_index_pair): EPW -1 thread-pair, 0 thread-per-element,
+        // otherwise the elements per warp pass of the lane-per-row (32 / nq) or generic (1) kernel, n_pass passes per patch
+        struct MetricLayout
+        {
+            int epw, n_pass;
+        };
+
+        // chooses the kernel, allocates the metric data and returns its layout
+        MetricLayout init_volume_common(VolumeOp & op, H1Space * fem, int nq, bool stiff, bool want_affine = false)
         {
             op.fem = fem;
             op.nb = fem->nb;
@@ -1514,58 +1585,35 @@ namespace cb200
             op.stiff = stiff;
             CB_REQUIRE(nq >= 1 && nq <= MAXQ, stiff ? "StiffnessMatrix::action does not support quadrature rules with more than 24 points."
                                                     : "MassMatrix error: quadrature rules with more than 32 points not yet supported.");
-            LaunchFn fn = stiff ? find_instance<true>(op.nb, nq) : find_instance<false>(op.nb, nq);
-            op.generic = force_generic || (fn == nullptr);
-            LaunchFn ft = stiff ? find_tpe_instance<true>(op.nb, nq) : find_tpe_instance<false>(op.nb, nq);
-            op.tpe = !op.generic && ft != nullptr && env_int("CUDDH_B200_TPE", 1) != 0;
-            op.nk = (stiff ? 3 : 1) * nq;
-            op.affine = want_affine && stiff && op.tpe && find_affine_instance(op.nb, nq) != nullptr && env_int("CUDDH_B200_AFFINE", 1) != 0 &&
-                        fem->all_affine();
-            const bool pair_affine = want_affine && stiff && env_int("CUDDH_B200_AFFINE", 1) != 0 && op.nb >= 6 && fem->all_affine();
-            LaunchFn fp = stiff ? find_pair_instance<true>(op.nb, nq, pair_affine) : find_pair_instance<false>(op.nb, nq);
-            op.pair = !op.generic && !op.tpe && fp != nullptr && env_int("CUDDH_B200_PAIR", 1) != 0;
-            if (op.pair) { // thread-pair layout: [row][pair of metric values][thread slot], see volume_action_pair / metric_index_pair
-                op.affine = pair_affine;
-                op.plan = &fem->get_plan_tpe();
-                // never with H1Space's own numbering and the default patch shape (the CUDDH_B200_TPE_PX / PY experiment knobs can change
-                // the latter): the lane-per-row kernel serves such a plan
-                if (op.plan->PE != 64 || !op.plan->interior_affine) {
-                    op.pair = false;
-                    op.affine = false;
-                }
+            const VolumeChoice k = select_volume_kernel(fem, op.nb, nq, stiff, want_affine);
+            op.kind = k.kind;
+            op.affine = k.affine;
+            op.launch = k.launch;
+            op.plan = k.plan;
+            const Plan & plan = *op.plan;
+            const int nki = stiff ? 3 : 1; // metric values per quadrature point
+            MetricLayout ml{0, 0};
+            size_t n_metric;
+            if (op.kind == VolumeKernel::ThreadPair) { // [row][pair of metric values][thread slot], see metric_index_pair
+                const int TA = (nq + 1) / 2, KR = (nki * TA + 1) & ~1;
+                ml.epw = -1;
+                n_metric = (size_t)plan.n_patches * (size_t)nq * KR * 128;
             }
-            if (op.pair) {
-                op.epw = -1;
-                op.lw = 0;
-                op.n_pass = 0;
-                const int TA = (nq + 1) / 2, KR = ((stiff ? 3 : 1) * TA + 1) & ~1;
-                if (op.affine)
-                    op.d_Gc.alloc((size_t)op.plan->n_patches * 3 * op.plan->PE);
-                else
-                    op.d_G.alloc((size_t)op.plan->n_patches * (size_t)nq * KR * 128);
+            else if (op.kind == VolumeKernel::ThreadPerElement) // [pair of metric values][element], see volume_action_ws
+                n_metric = (size_t)plan.n_patches * (size_t)(nq * ((nki * nq + 1) & ~1)) * plan.PE;
+            else { // lane-major per warp pass, see metric_index
+                ml.epw = op.kind == VolumeKernel::Generic ? 1 : 32 / nq;
+                ml.n_pass = (plan.PE + ml.epw - 1) / ml.epw;
+                n_metric = (size_t)plan.n_patches * ml.n_pass * (nki * nq) * (ml.epw * nq);
             }
-            else if (op.tpe) { // thread-per-element layout: [pair of metric values][element], see volume_action_ws
-                op.plan = &fem->get_plan_tpe();
-                op.epw = 0;
-                op.lw = 0;
-                op.n_pass = 0;
-                const int KR = (op.nk + 1) & ~1;
-                if (op.affine)
-                    op.d_Gc.alloc((size_t)op.plan->n_patches * 3 * op.plan->PE);
-                else
-                    op.d_G.alloc((size_t)op.plan->n_patches * (size_t)(nq * KR) * op.plan->PE);
-            }
-            else {
-                op.plan = &fem->get_plan();
-                op.epw = op.generic ? 1 : 32 / nq;
-                op.lw = op.epw * nq;
-                op.n_pass = (op.plan->PE + op.epw - 1) / op.epw;
-                op.d_G.alloc((size_t)op.plan->n_patches * op.n_pass * op.nk * op.lw);
-            }
-            Plan & plan = *op.plan;
+            if (op.affine)
+                op.d_Gc.alloc((size_t)plan.n_patches * 3 * plan.PE);
+            else
+                op.d_G.alloc(n_metric);
             op.d_partial.alloc((size_t)std::max<int64_t>(plan.n_slots_total, 1));
             if (op.d_G.n)
                 CB_CUDA(cudaMemset(op.d_G.p, 0, op.d_G.n * sizeof(double)));
+            return ml;
         }
     } // namespace
 
@@ -1575,7 +1623,7 @@ namespace cb200
         if (nq <= 0)
             nq = fem->nb + 1; // mesh.max_element_order() (=1) + n_basis, StiffnessMatrix.cpp:45
         CB_REQUIRE(nq <= 24, "StiffnessMatrix::action does not support quadrature rules with more than 24 points.");
-        init_volume_common(*op, fem, nq, true, getenv("CUDDH_B200_FORCE_GENERIC") != nullptr, quad_type == GAUSS_LEGENDRE);
+        const MetricLayout ml = init_volume_common(*op, fem, nq, true, quad_type == GAUSS_LEGENDRE);
         std::vector<double> xq(nq), wq(nq);
         quadrature_rule(nq, quad_type, xq.data(), wq.data());
         op->wq = wq;
@@ -1593,7 +1641,7 @@ namespace cb200
         if (op->affine)
             setup_stiffness_affine_kernel<<<blocks_for(n_slots, 256), 256>>>(n_slots, plan.PE, plan.d_slot_elem.p, fem->device_corners(), op->d_Gc.p);
         else
-            setup_stiffness_kernel<<<blocks_for(n_slots * nq * nq, 256), 256>>>(n_slots, plan.PE, nq, op->epw, op->n_pass, plan.d_slot_elem.p,
+            setup_stiffness_kernel<<<blocks_for(n_slots * nq * nq, 256), 256>>>(n_slots, plan.PE, nq, ml.epw, ml.n_pass, plan.d_slot_elem.p,
                                                                                 fem->device_corners(), d_x.p, d_w.p, op->d_G.p);
         CB_LAUNCHED();
         CB_CUDA(cudaDeviceSynchronize());
@@ -1605,7 +1653,7 @@ namespace cb200
         std::unique_ptr<VolumeOp> op(new VolumeOp);
         if (nq <= 0) // MassMatrix.cpp:74 (unweighted) / :108 (weighted)
             nq = d_coef ? (1 + 3 * fem->nb / 2 + 1) : (fem->nb + 1);
-        init_volume_common(*op, fem, nq, false, getenv("CUDDH_B200_FORCE_GENERIC") != nullptr);
+        const MetricLayout ml = init_volume_common(*op, fem, nq, false);
         std::vector<double> xq(nq), wq(nq);
         quadrature_rule(nq, GAUSS_LEGENDRE, xq.data(), wq.data());
         op->P.resize((size_t)nq * fem->nb);
@@ -1616,7 +1664,7 @@ namespace cb200
         d_w.upload(wq);
         Plan & plan = *op->plan;
         const int64_t n_slots = plan.n_patches * plan.PE;
-        setup_mass_kernel<<<blocks_for(n_slots * nq * nq, 256), 256>>>(n_slots, plan.PE, fem->nb, nq, op->epw, op->n_pass, plan.d_slot_elem.p,
+        setup_mass_kernel<<<blocks_for(n_slots * nq * nq, 256), 256>>>(n_slots, plan.PE, fem->nb, nq, ml.epw, ml.n_pass, plan.d_slot_elem.p,
                                                                        fem->device_corners(), fem->device_I(), d_coef, op->d_P.p, d_x.p,
                                                                        d_w.p, op->d_G.p);
         CB_LAUNCHED();
@@ -1990,16 +2038,9 @@ namespace cb200
         op->S = make_stiffness(fem, 0, GAUSS_LEGENDRE);
         op->M = make_mass(fem, d_a2, 0);
         op->H = make_facemass(fs, d_a, 0);
-        op->fused = op->S->tpe && op->M->tpe && op->S->plan == op->M->plan &&
-                    find_fused_instance(op->S->nb, op->S->nq, op->M->nq, op->S->affine) != nullptr &&
-                    env_int("CUDDH_B200_FUSED", 1) != 0;
-        // n_basis 6-8: the thread-pair kernel runs S - w^2 M of one field per launch (two launches per apply)
-        op->fused_pair = op->S->pair && op->M->pair && op->S->plan == op->M->plan &&
-                         find_fused_pair_instance(op->S->nb, op->S->nq, op->M->nq, op->S->affine) != nullptr &&
-                         env_int("CUDDH_B200_FUSED", 1) != 0;
-        op->fused = op->fused || op->fused_pair;
+        op->fused = select_fused_kernel(*op->S, *op->M);
         if (op->fused)
-            op->d_partial2.alloc(2 * (size_t)std::max<int64_t>(op->S->plan->n_slots_total, 1));
+            op->d_partial2.alloc(2 * (size_t)partial_stride(*op));
         return op;
     }
 
@@ -2013,52 +2054,14 @@ namespace cb200
         double * Au = y;
         double * Av = y + n;
         if (fused) {
-            // one warp-specialised kernel walks (patch, field) units: S and M share the gather, the index lists and the
-            // assembly, the sign of the second block row is applied on write: 3 launches instead of 11 + 4 memsets
-            Plan & plan = *S->plan;
-            PlanDev pd{plan.d_hdr.p, plan.d_gid.p, plan.d_slot.p, plan.d_L.p, plan.d_cptr.p, plan.d_cent.p, plan.PE, plan.d_Ig.p,
-                       reinterpret_cast<const uint2 *>(plan.d_cent4.p), plan.d_target.p};
-            WsArgs a{};
-            a.G1 = reinterpret_cast<const double2 *>(S->d_G.p);
-            a.G2 = reinterpret_cast<const double2 *>(M->d_G.p);
-            a.Gc = S->d_Gc.p;
-            a.x = x;
-            a.y = y;
-            a.partial = d_partial2.p;
-            a.x_stride = a.y_stride = n;
-            a.partial_stride = std::max<int64_t>(plan.n_slots_total, 1);
-            a.c[0] = 1.0;
-            a.c[1] = -1.0;
-            a.msc = -omega * omega;
-            a.accumulate = 0;
-            a.n_patches = (int)plan.n_patches;
-            a.n_fields = 2;
-            if ((phases & 1) && !fused_pair)
-                find_fused_instance(S->nb, S->nq, M->nq, S->affine)(*S, M.get(), pd, plan, a, s);
-            if ((phases & 1) && fused_pair) {
-                FusedPairFn fn = find_fused_pair_instance(S->nb, S->nq, M->nq, S->affine);
-                for (int f = 0; f < 2; ++f) {
-                    PairArgs pa{};
-                    pa.G = reinterpret_cast<const double2 *>(S->d_G.p);
-                    pa.G2 = reinterpret_cast<const double2 *>(M->d_G.p);
-                    pa.Gc = S->d_Gc.p;
-                    pa.x = x + f * n;
-                    pa.y = y + f * n;
-                    pa.partial = d_partial2.p + f * a.partial_stride;
-                    pa.c = a.c[f];
-                    pa.msc = a.msc;
-                    pa.accumulate = 0;
-                    fn(*S, M.get(), pd, plan, pa, s);
-                }
+            // one volume kernel walks (patch, field) units: S and M share the gather, the index lists and the assembly, the
+            // sign of the second block row is applied on write: 3 launches instead of 11 + 4 memsets
+            if (phases & 1)
+                fused(*this, x, y, s);
+            if (phases & 2) {
+                assemble_shared_fields(*this, y, s);
+                H->apply_h1_pair(-omega, x, y, n, s); // Au -= w H v ; Av -= w H u in one launch
             }
-            if (!(phases & 2))
-                return;
-            if (plan.n_shared > 0) {
-                assemble_shared_fields_kernel<<<dim3(blocks_for(plan.n_shared, 256), 2), 256, 0, s>>>(
-                    plan.n_shared, plan.d_sh_gid.p, plan.d_sh_ptr.p, d_partial2.p, a.partial_stride, y, n, 1.0, -1.0);
-                CB_LAUNCHED();
-            }
-            H->apply_h1_pair(-omega, x, y, n, s); // Au -= w H v ; Av -= w H u in one launch
             return;
         }
         // 7 launches + 4 tiny assembly passes instead of the reference's 11 kernels + 4 memsets.
@@ -2083,12 +2086,7 @@ namespace cb200
         if (fused) {
             // volume kernel + shared-DOF pass, then ONE launch for both face terms and the pack of the interface rows
             apply(x, y, s, 1);
-            Plan & plan = *S->plan;
-            if (plan.n_shared > 0) {
-                assemble_shared_fields_kernel<<<dim3(blocks_for(plan.n_shared, 256), 2), 256, 0, s>>>(
-                    plan.n_shared, plan.d_sh_gid.p, plan.d_sh_ptr.p, d_partial2.p, std::max<int64_t>(plan.n_slots_total, 1), y, fem->ndof, 1.0, -1.0);
-                CB_LAUNCHED();
-            }
+            assemble_shared_fields(*this, y, s);
             ++halo.epoch;
             H->apply_h1_pair(-omega, x, y, fem->ndof, s, &halo);
             if (!halo.peer)

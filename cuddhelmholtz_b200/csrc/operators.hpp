@@ -9,6 +9,9 @@ namespace cb200
     struct SlabHalo;
     struct HelmholtzOp;
 
+    // kernel family of a volume operator, chosen once at construction (select_volume_kernel in operators.cu)
+    enum class VolumeKernel { Generic, LanePerRow, ThreadPerElement, ThreadPair };
+
     // y = (accumulate ? y : 0) + c * A x  for a patch-planned volume operator
     struct VolumeOp
     {
@@ -22,10 +25,8 @@ namespace cb200
         DevBuf<double> d_Gc;          // affine stiffness: per patch (3, PE) element constants gA, gB, gC instead of d_G
         bool affine = false;          // stiffness on a mesh whose elements are all parallelograms: metric = w_i w_j * per-element constants
         DevBuf<double> d_partial;     // partial sums of patch-boundary DOFs
-        int epw = 0, lw = 0, n_pass = 0, nk = 0;  // layout constants (see operators.cu)
-        bool generic = false;
-        bool tpe = false;             // thread-per-element kernel + node-major plan (n_basis <= 5)
-        bool pair = false;            // thread-pair-per-element kernel + node-major plan of 64-element patches (n_basis 6-9)
+        VolumeKernel kind = VolumeKernel::Generic; // and the template instance that runs it (null: Generic)
+        void (*launch)(const VolumeOp &, double c, int accumulate, const double * x, double * y, cudaStream_t s) = nullptr;
         Plan * plan = nullptr;        // the assembly plan this operator was laid out for (owned by fem)
 
         // phases: bit 0 = patch kernel, bit 1 = shared-DOF assembly pass (3 = the full action)
@@ -122,8 +123,8 @@ namespace cb200
         std::unique_ptr<VolumeOp> S, M;
         std::unique_ptr<FaceMassOp> H;
         DevBuf<double> d_partial2;    // fused path: partial sums of patch-boundary DOFs for both fields
-        bool fused = false;           // S - omega^2 M on u and v in one warp-specialised kernel (n_basis <= 5), or per field (fused_pair)
-        bool fused_pair = false;      // n_basis 6-8: the thread-pair kernel with both phases, one launch per field
+        // fused path: S - omega^2 M on u and v, one launch for both fields (n_basis <= 5) or one per field (6-9); null: one by one
+        void (*fused)(const HelmholtzOp &, const double * x, double * y, cudaStream_t s) = nullptr;
         // phases (fused path only): bit 0 = the fused volume kernel, bit 1 = shared-DOF assembly + face terms
         void apply(const double * x, double * y, cudaStream_t s, int phases = 3);
         // the apply of one slab of a partitioned mesh: local apply, interface rows packed inside the face-mass launch,
