@@ -13,6 +13,7 @@ streams here) or raw device addresses (int).
     gmres(n, x, A, b, [P,] m, maxit, tol,..)   gmres(n, x, A, b, m, maxit, tol, P=None, ...)
     DDH(omega, h_a, fem, nx, ny)               DDH(omega, h_a, fem, nx, ny, block=16)
     (new) DDHTransfer(ddh)                     DDHTransfer(ddh, max_bytes=0): the same operator with T assembled
+    (new) many sources at once                 DDHTransfer.action_batch(X, Y), gmres_batch(n, X, A, B, m, maxit, tol)
 """
 import ctypes as C
 import numpy as np
@@ -59,6 +60,20 @@ def _np(a, dtype):
 
 def _vp(a):
     return a.ctypes.data_as(C.c_void_p)
+
+
+def _rows(X, n=None):
+    """(k, host array of the k row addresses) of a float32 CUDA tensor of shape (k, n) with contiguous rows"""
+    import torch
+    if not isinstance(X, torch.Tensor) or not X.is_cuda or X.dtype != torch.float32 or X.dim() != 2:
+        raise capi.CuddhError("expected a float32 CUDA tensor of shape (k, n)")
+    if X.shape[1] > 1 and X.stride(1) != 1:
+        raise capi.CuddhError("expected contiguous rows")
+    if n is not None and X.shape[1] != n:
+        raise capi.CuddhError("expected rows of length %d, got %d" % (n, X.shape[1]))
+    k = X.shape[0]
+    base, step = X.data_ptr(), X.stride(0) * X.element_size()
+    return k, (C.c_void_p * max(k, 1))(*[base + j * step for j in range(k)])
 
 
 class QuadratureRule:
@@ -506,6 +521,28 @@ def _callback(A, kind):
     return C.cast(cb, C.c_void_p), None, cb
 
 
+def _callback_batch(A):
+    """(function pointer, ctx, keepalive) of a batched operator, as _callback: library objects with _as_apply_batch use the
+    in-library trampoline, any object with .action_batch(x_ptrs, y_ptrs) (lists of raw device addresses, one per active system)
+    is wrapped in a ctypes callback whose exceptions abort the solve and are re-raised after it."""
+    if hasattr(A, "_as_apply_batch"):
+        fn, ctx = A._as_apply_batch()
+        return fn, ctx, None
+    if not hasattr(A, "action_batch"):
+        raise capi.CuddhError("gmres_batch: the operator needs _as_apply_batch or .action_batch(x_ptrs, y_ptrs)")
+
+    def tramp(_ctx, k, x, y, _stream):
+        try:
+            A.action_batch([int(x[j]) for j in range(k)], [int(y[j]) for j in range(k)])
+            return 0
+        except BaseException as e:
+            _callback_error.append(e)
+            return -7
+
+    cb = capi.APPLY_BATCH_F(tramp)
+    return C.cast(cb, C.c_void_p), None, cb
+
+
 MGS, CGS2 = 0, 1
 
 
@@ -540,6 +577,31 @@ def gmres(n, x, A, b, m, maxit, tol=None, P=None, verbose=0, max_seconds=6 * 60 
         raise _callback_error.pop()
     check(rc)
     return SolverOut(so, res, tim, st)
+
+
+def gmres_batch(n, X, A, B, m, maxit, tol=1e-4, max_seconds=6 * 60 * 60):
+    """k independent FP32 GMRES(m) solves A X[j] = B[j] in lockstep (k <= 32): one batched operator application and one host sync
+    per Arnoldi step for all systems still iterating. X, B: float32 CUDA tensors of shape (k, n) with contiguous rows; X holds
+    the initial guesses and receives the solutions. A: DDHTransfer, or any object with .action_batch(x_ptrs, y_ptrs), which is
+    handed only the active systems. MGS arithmetic: each system's solution, residual norms, num_iter and num_matvec are bitwise
+    those of gmres(n, X[j], A, B[j], m, maxit, tol, orth=MGS). max_seconds limits the whole batch. Returns one SolverOut per system."""
+    k, xp = _rows(X, n)
+    kb, bp = _rows(B, n)
+    if kb != k:
+        raise capi.CuddhError("gmres_batch: X and B must have the same number of rows")
+    fa, ca, keep = _callback_batch(A)
+    cap = maxit + 2
+    rows = max(k, 1)
+    res = np.zeros((rows, cap))
+    tim = np.zeros((rows, cap))
+    so = (capi.SolverOut * rows)()
+    del _callback_error[:]
+    rc = load().cuddh_b200_gmres_f_batch(n, k, xp, fa, ca, bp, m, maxit, float(tol), float(max_seconds), so, _vp(res), _vp(tim), cap,
+                                         _stream())
+    if _callback_error:
+        raise _callback_error.pop()
+    check(rc)
+    return [SolverOut(so[j], res[j], tim[j]) for j in range(k)]
 
 
 def set_option(name, value):
@@ -678,6 +740,16 @@ class DDHTransfer:
     def action(self, x, y):
         check(load().cuddh_b200_ddh_transfer_action(self._h, _ptr(x), _ptr(y), _stream()))
 
+    def action_batch(self, X, Y):
+        """Y[j] = X[j] - T X[j] for the k rows of float32 CUDA tensors of shape (k, n) with contiguous rows, 1 <= k <= 32. Row j is
+        bitwise action(X[j]); the blocks stream once for up to 16 rows. Overlapping outputs (with any input or each other) raise."""
+        n = self.size()
+        k, xp = _rows(X, n)
+        ky, yp = _rows(Y, n)
+        if ky != k:
+            raise capi.CuddhError("action_batch: X and Y must have the same number of rows")
+        check(load().cuddh_b200_ddh_transfer_action_batch(self._h, k, xp, yp, _stream()))
+
     def rhs(self, f, b):
         self.ddh.rhs(f, b)
 
@@ -704,6 +776,9 @@ class DDHTransfer:
 
     def _as_apply(self):
         return C.cast(load().cuddh_b200_ddh_transfer_as_apply, C.c_void_p), self._h
+
+    def _as_apply_batch(self):
+        return C.cast(load().cuddh_b200_ddh_transfer_as_apply_batch, C.c_void_p), self._h
 
 
 class DDHPreconditioner:

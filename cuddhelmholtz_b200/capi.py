@@ -14,6 +14,8 @@ c_dp = C.c_void_p  # device or host pointers are passed as raw addresses
 # cuddh_apply_{d,f}_fn: int (*)(void* ctx, const T* x, T* y, void* stream); non-zero aborts the solve
 APPLY_D = C.CFUNCTYPE(C.c_int, c_vp, c_vp, c_vp, c_vp)
 APPLY_F = C.CFUNCTYPE(C.c_int, c_vp, c_vp, c_vp, c_vp)
+# cuddh_apply_batch_f_fn: int (*)(void* ctx, int k, const float* const* x, float* const* y, void* stream); x, y: host pointer arrays
+APPLY_BATCH_F = C.CFUNCTYPE(C.c_int, c_vp, C.c_int, C.POINTER(c_vp), C.POINTER(c_vp), c_vp)
 
 
 class SolverOut(C.Structure):
@@ -170,6 +172,10 @@ def _proto(lib):
         "cuddh_b200_ddh_transfer_as_apply": (C.c_int, [c_vp, c_dp, c_dp, c_vp]),
         "cuddh_b200_ddh_transfer_info": (C.c_int, [c_vp, c_vp]),
         "cuddh_b200_ddh_transfer_get_block": (C.c_int, [c_vp, C.c_int, c_vp]),
+        "cuddh_b200_ddh_transfer_action_batch": (C.c_int, [c_vp, C.c_int, c_vp, c_vp, c_vp]),
+        "cuddh_b200_ddh_transfer_as_apply_batch": (C.c_int, [c_vp, C.c_int, c_vp, c_vp, c_vp]),
+        "cuddh_b200_gmres_f_batch": (C.c_int, [c_i64, C.c_int, c_vp, c_vp, c_vp, c_vp, C.c_int, C.c_int, C.c_float, C.c_double,
+                                               c_vp, c_vp, c_vp, C.c_int, c_vp]),
     }
     for name, (res, args) in sig.items():
         fn = getattr(lib, name)

@@ -1067,4 +1067,46 @@ int cuddh_b200_ddh_transfer_get_block(cuddh_ddh_transfer_t h, int dom, float * h
     CB_CATCH
 }
 
+// ---- many right-hand sides ----
+int cuddh_b200_ddh_transfer_action_batch(cuddh_ddh_transfer_t h, int k, const float * const * x, float * const * y, void * stream)
+{
+    CB_TRY
+    DDHTransfer::check_batch_args(k, x, y);
+    CB_REQUIRE(h != nullptr, "ddh_transfer_action_batch: null handle");
+    h->t->action_batch(k, x, y, S(stream));
+    CB_CATCH
+}
+int cuddh_b200_ddh_transfer_as_apply_batch(void * h, int k, const float * const * x, float * const * y, void * stream)
+{
+    return cuddh_b200_ddh_transfer_action_batch((cuddh_ddh_transfer_t)h, k, x, y, stream);
+}
+} // extern "C"
+namespace
+{
+    struct UserApplyBatch // the C ABI batched callback (void* stream) behind the internal one
+    {
+        cuddh_apply_batch_f_fn fn;
+        void * ctx;
+        static int apply(void * self, int k, const float * const * x, float * const * y, cudaStream_t st)
+        {
+            auto * u = (UserApplyBatch *)self;
+            return u->fn(u->ctx, k, x, y, (void *)st);
+        }
+    };
+} // namespace
+extern "C" {
+int cuddh_b200_gmres_f_batch(int64_t n, int k, float * const * x, cuddh_apply_batch_f_fn A, void * A_ctx, const float * const * b, int m,
+                             int maxit, float tol, double max_seconds, cuddh_solver_out * out, double * h_res_norm, double * h_time,
+                             int cap, void * stream)
+{
+    CB_TRY
+    UserApplyBatch ua{A, A_ctx};
+    const std::vector<GmresResult> r =
+        gmres_batch<float>(n, k, x, A ? &UserApplyBatch::apply : nullptr, &ua, b, m, maxit, tol, max_seconds, S(stream));
+    for (int j = 0; j < k; ++j)
+        fill_out(r[j], out ? out + j : nullptr, h_res_norm ? h_res_norm + (size_t)j * std::max(cap, 0) : nullptr,
+                 h_time ? h_time + (size_t)j * std::max(cap, 0) : nullptr, cap);
+    CB_CATCH
+}
+
 } // extern "C"

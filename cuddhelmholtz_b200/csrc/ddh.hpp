@@ -114,6 +114,12 @@ namespace cb200
         int64_t block_bytes() const { return (int64_t)slots.two_f * slots.two_f * slots.n_domains * (int64_t)sizeof(float); }
         int64_t bytes_per_action() const;   // blocks + maps + gathered inputs + written outputs + orphan copies
         void action(const float * x, float * y, cudaStream_t s); // y = x - T x; x and y must not overlap
+        // y_j = x_j - T x_j for j < k (1 <= k <= KMAX); x, y: HOST arrays of k device pointers. No y_j may overlap any x_i or another
+        // y_i. Row j is bitwise action(x_j). Passes of up to 16 vectors stream the blocks once each; a pass of one or two vectors
+        // runs the single-vector kernel per vector. At most ceil(k / 16) + 1 launches.
+        static constexpr int KMAX = 32;
+        void action_batch(int k, const float * const * x, float * const * y, cudaStream_t s);
+        static void check_batch_args(int k, const void * x, const void * y); // k range, null arrays (host only, no CUDA call)
         void get_block(int dom, float * h_out) const;            // host copy of M_dom (2F x 2F, column-major)
     };
 

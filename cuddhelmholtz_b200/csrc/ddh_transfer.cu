@@ -154,6 +154,95 @@ namespace cb200
             if (o.w >= 0) y[o.w] = __ldg(x + o.w) - r3;
         }
 
+        // Vectors per pass of the batched action. 16 keeps 64 FP32 accumulators per thread (no spills, two CTAs per SM) and turns
+        // every 16-byte block load into 64 FMAs, which puts FP32 issue and the block stream of an action at about the same time.
+        constexpr int TR_KB = 16;
+
+        // the pointers of one pass, passed by value (no device copy per call)
+        struct TransferBatchArgs
+        {
+            const float * x[TR_KB];
+            float * y[TR_KB];
+        };
+
+        // The action of ddh_transfer_action_kernel on nv <= KB vectors at once: the same CTA / subdomain shape, the gathered inputs
+        // laid out [sub][column][vec] so that the KB values of one column are KB / 4 broadcast 128-bit shared loads, and every
+        // block column streamed once for all vectors. Each accumulator is the single-vector kernel's chain (fmaf over ascending
+        // columns from 0.0f), so column j of the result is bitwise ddh_transfer_action_kernel(x_j).
+        template <int TF, int KB>
+        __global__ void __launch_bounds__(TR_THREADS, 2)
+        ddh_transfer_action_batch_kernel(const float * __restrict__ M, const int * __restrict__ in, const int * __restrict__ out,
+                                         const int * __restrict__ orphans, const int n_orphans, const TransferBatchArgs a, const int nv,
+                                         const int n_domains, const int n_dom_ctas)
+        {
+            using SH = TransferShape<TF>;
+            constexpr int Q = SH::Q, SPB = SH::SPB, NT = SH::NT, KV = KB / 4;
+            static_assert(KB % 4 == 0 && KB <= TR_KB, "KB: a multiple of 4, at most TR_KB");
+            extern __shared__ float4 s_xb[]; // (SPB, TF, KV) float4
+
+            if ((int)blockIdx.x >= n_dom_ctas) { // slots no subdomain writes: y = x
+                const int i = ((int)blockIdx.x - n_dom_ctas) * NT + (int)threadIdx.x;
+                if (i < n_orphans) {
+                    const int o = __ldg(orphans + i);
+#pragma unroll
+                    for (int v = 0; v < KB; ++v)
+                        if (v < nv)
+                            a.y[v][o] = __ldg(a.x[v] + o);
+                }
+                return;
+            }
+            const int dom0 = blockIdx.x * SPB;
+            const int nloc = min(SPB, n_domains - dom0);
+            const int * inb = in + (size_t)dom0 * TF;
+            float * sx = reinterpret_cast<float *>(s_xb);
+            for (int t = threadIdx.x; t < nloc * TF; t += NT) { // t = sub * TF + column
+                const int s = __ldg(inb + t);
+#pragma unroll
+                for (int v = 0; v < KB; ++v)
+                    sx[t * KB + v] = (s >= 0 && v < nv) ? __ldg(a.x[v] + s) : 0.0f;
+            }
+            __syncthreads();
+            const int sub = threadIdx.x / Q, q = threadIdx.x % Q;
+            if (sub >= nloc)
+                return;
+            const int dom = dom0 + sub;
+            const float4 * Mp = reinterpret_cast<const float4 *>(M + (size_t)dom * TF * TF) + q;
+            const float4 * xs = s_xb + sub * TF * KV;
+            const uint64_t pol = evict_first_policy();
+            float r[KB][4];
+#pragma unroll
+            for (int v = 0; v < KB; ++v)
+                r[v][0] = r[v][1] = r[v][2] = r[v][3] = 0.0f;
+#pragma unroll 4
+            for (int k = 0; k < TF; ++k) {
+                const float4 m = ld_stream(Mp + (size_t)k * Q, pol);
+#pragma unroll
+                for (int g = 0; g < KV; ++g) {
+                    const float4 xv = xs[k * KV + g];
+                    const float xk[4] = {xv.x, xv.y, xv.z, xv.w};
+#pragma unroll
+                    for (int c = 0; c < 4; ++c) {
+                        float * rv = r[4 * g + c];
+                        rv[0] = fmaf(m.x, xk[c], rv[0]);
+                        rv[1] = fmaf(m.y, xk[c], rv[1]);
+                        rv[2] = fmaf(m.z, xk[c], rv[2]);
+                        rv[3] = fmaf(m.w, xk[c], rv[3]);
+                    }
+                }
+            }
+            const int4 o = __ldg(reinterpret_cast<const int4 *>(out + (size_t)dom * TF) + q);
+#pragma unroll
+            for (int v = 0; v < KB; ++v)
+                if (v < nv) {
+                    const float * xv = a.x[v];
+                    float * yv = a.y[v];
+                    if (o.x >= 0) yv[o.x] = __ldg(xv + o.x) - r[v][0];
+                    if (o.y >= 0) yv[o.y] = __ldg(xv + o.y) - r[v][1];
+                    if (o.z >= 0) yv[o.z] = __ldg(xv + o.z) - r[v][2];
+                    if (o.w >= 0) yv[o.w] = __ldg(xv + o.w) - r[v][3];
+                }
+        }
+
         // probe k: local input k of every subdomain to 1, input k - 1 of the previous probe back to 0 (no slot has two readers,
         // so the two writes never meet)
         __global__ void ddh_transfer_probe_scatter(const int * __restrict__ in, const int TF, const int k, const int n_domains,
@@ -196,6 +285,46 @@ namespace cb200
             ddh_transfer_action_kernel<TF><<<dom_ctas + orph_ctas, SH::NT, 0, s>>>(T.d_M.p, T.d_in.p, T.d_out.p, T.d_orphans.p, no, x, y, nd,
                                                                                  dom_ctas);
             CB_LAUNCHED();
+        }
+
+        // Passes of at most this many vectors run the single-vector kernel once per vector (bitwise the same rows): a pass of the
+        // 16-wide kernel streams the blocks at about 2.8 TB/s against 6.7 TB/s for the single-vector kernel (512^2, one B200), so
+        // up to two vectors are faster one at a time.
+        constexpr int TR_SINGLE_MAX = 2;
+
+        // one launch per pass of up to TR_KB vectors (one per vector for passes of at most TR_SINGLE_MAX)
+        template <int TF>
+        void launch_action_batch(const DDHTransfer & T, int k, const float * const * x, float * const * y, cudaStream_t s)
+        {
+            using SH = TransferShape<TF>;
+            constexpr size_t smem = (size_t)SH::SPB * TF * TR_KB * sizeof(float);
+            static std::atomic<uint64_t> attr_set{0}; // per device ordinal: dynamic shared-memory limit raised
+            int dev = 0;
+            CB_CUDA(cudaGetDevice(&dev));
+            CB_REQUIRE(dev >= 0 && dev < 64, "device ordinal out of range");
+            auto kern = ddh_transfer_action_batch_kernel<TF, TR_KB>;
+            if (!(attr_set.load() >> dev & 1)) {
+                CB_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+                attr_set.fetch_or(uint64_t(1) << dev);
+            }
+            const int nd = T.slots.n_domains, no = (int)T.slots.orphans.size();
+            const int dom_ctas = (nd + SH::SPB - 1) / SH::SPB;
+            const int orph_ctas = (no + SH::NT - 1) / SH::NT;
+            for (int j0 = 0; j0 < k; j0 += TR_KB) {
+                const int nv = std::min(TR_KB, k - j0);
+                if (nv <= TR_SINGLE_MAX) {
+                    for (int v = 0; v < nv; ++v)
+                        launch_action<TF>(T, x[j0 + v], y[j0 + v], s);
+                    continue;
+                }
+                TransferBatchArgs a{};
+                for (int v = 0; v < nv; ++v) {
+                    a.x[v] = x[j0 + v];
+                    a.y[v] = y[j0 + v];
+                }
+                kern<<<dom_ctas + orph_ctas, SH::NT, smem, s>>>(T.d_M.p, T.d_in.p, T.d_out.p, T.d_orphans.p, no, a, nv, nd, dom_ctas);
+                CB_LAUNCHED();
+            }
         }
     } // namespace
 
@@ -275,6 +404,34 @@ namespace cb200
         case 112: launch_action<112>(*this, x, y, s); break;
         case 192: launch_action<192>(*this, x, y, s); break;
         case 224: launch_action<224>(*this, x, y, s); break;
+        default: throw Error(-1, "DDH transfer: no action kernel for this n_basis / block");
+        }
+    }
+
+    void DDHTransfer::check_batch_args(int k, const void * x, const void * y)
+    {
+        CB_REQUIRE(k >= 1 && k <= KMAX, "DDH transfer action_batch: k must be in [1, " + std::to_string(KMAX) + "]");
+        CB_REQUIRE(x != nullptr && y != nullptr, "DDH transfer action_batch: null pointer array");
+    }
+
+    void DDHTransfer::action_batch(int k, const float * const * x, float * const * y, cudaStream_t s)
+    {
+        NvtxRange nvtx_("cuddh::DDHTransfer::action_batch");
+        check_batch_args(k, x, y);
+        const int64_t n = 2 * slots.n_lambda;
+        for (int j = 0; j < k; ++j)
+            CB_REQUIRE(x[j] != nullptr && y[j] != nullptr, "DDH transfer action_batch: null vector pointer");
+        auto overlap = [n](const float * a, const float * b) { return a < b + n && b < a + n; };
+        for (int j = 0; j < k; ++j)
+            for (int i = 0; i < k; ++i)
+                if (overlap(y[j], x[i]) || (i != j && overlap(y[j], y[i])))
+                    throw Error(-1, "DDH transfer action_batch: output " + std::to_string(j) + " overlaps " + (i != j && overlap(y[j], y[i]) ? "output " : "input ") +
+                                        std::to_string(i));
+        switch (slots.two_f) {
+        case 96: launch_action_batch<96>(*this, k, x, y, s); break;
+        case 112: launch_action_batch<112>(*this, k, x, y, s); break;
+        case 192: launch_action_batch<192>(*this, k, x, y, s); break;
+        case 224: launch_action_batch<224>(*this, k, x, y, s); break;
         default: throw Error(-1, "DDH transfer: no action kernel for this n_basis / block");
         }
     }

@@ -127,10 +127,10 @@ namespace cb200
             }
         }
 
+        // body of reduce_kernel, shared with the batched solve (one system per grid row: same partition, same tree)
         template <typename T, int MODE> // MODE 0: x.y   1: (x-y)^2
-        __global__ void __launch_bounds__(RED_THREADS)
-        reduce_kernel(const int64_t n, const T * __restrict__ x, const T * __restrict__ y, T * __restrict__ partials,
-                      unsigned * __restrict__ ticket, T * __restrict__ result, const int take_sqrt)
+        __device__ __forceinline__ void reduce_block(const int64_t n, const T * __restrict__ x, const T * __restrict__ y, T * __restrict__ partials,
+                                                     unsigned * __restrict__ ticket, T * __restrict__ result, const int take_sqrt)
         {
             T acc = 0;
             const int64_t stride = (int64_t)gridDim.x * RED_THREADS;
@@ -145,14 +145,22 @@ namespace cb200
             block_finish(acc, partials, ticket, result, take_sqrt != 0);
         }
 
+        template <typename T, int MODE>
+        __global__ void __launch_bounds__(RED_THREADS)
+        reduce_kernel(const int64_t n, const T * __restrict__ x, const T * __restrict__ y, T * __restrict__ partials,
+                      unsigned * __restrict__ ticket, T * __restrict__ result, const int take_sqrt)
+        {
+            reduce_block<T, MODE>(n, x, y, partials, ticket, result, take_sqrt);
+        }
+
         // fused MGS step on 16-byte-aligned basis columns: w -= h[prev] * vprev (if vprev), then <w, vnext> -> hout
         // (vnext == null: <w, w>, square root on the device unless the result still has to be summed over ranks).
         // Inner products count the entries with mask != 0 (mask == null: all).
+        // (body of mgs_step_kernel, shared with the batched solve)
         template <typename T>
-        __global__ void __launch_bounds__(RED_THREADS)
-        mgs_step_kernel(const int64_t n, T * __restrict__ w, const T * __restrict__ vprev, const T * __restrict__ vnext,
-                        const T * __restrict__ hprev, const unsigned char * __restrict__ mask, T * __restrict__ partials,
-                        unsigned * __restrict__ ticket, T * __restrict__ hout, const int take_sqrt)
+        __device__ __forceinline__ void mgs_step_block(const int64_t n, T * __restrict__ w, const T * __restrict__ vprev, const T * __restrict__ vnext,
+                                                       const T * __restrict__ hprev, const unsigned char * __restrict__ mask, T * __restrict__ partials,
+                                                       unsigned * __restrict__ ticket, T * __restrict__ hout, const int take_sqrt)
         {
             using P = Pack<T>;
             constexpr int N = P::N;
@@ -198,6 +206,15 @@ namespace cb200
                     acc = fma(wi, vnext ? vnext[i] : wi, acc);
             }
             block_finish(acc, partials, ticket, hout, take_sqrt != 0);
+        }
+
+        template <typename T>
+        __global__ void __launch_bounds__(RED_THREADS)
+        mgs_step_kernel(const int64_t n, T * __restrict__ w, const T * __restrict__ vprev, const T * __restrict__ vnext,
+                        const T * __restrict__ hprev, const unsigned char * __restrict__ mask, T * __restrict__ partials,
+                        unsigned * __restrict__ ticket, T * __restrict__ hout, const int take_sqrt)
+        {
+            mgs_step_block(n, w, vprev, vnext, hprev, mask, partials, ticket, hout, take_sqrt);
         }
 
         // CGS pass 1: partial sums of <w, v_j> for the JT basis columns of CTA row blockIdx.y (and of <w, w> in row 0), FP64
@@ -340,12 +357,33 @@ namespace cb200
             }
         }
 
+        // element bodies shared by the single and the batched kernels (same expression, same contraction)
+        template <typename T>
+        __device__ __forceinline__ void axpby_at(const int64_t i, const T a, const T * __restrict__ x, const T b, T * __restrict__ y)
+        {
+            y[i] = a * x[i] + b * y[i];
+        }
+        template <typename T>
+        __device__ __forceinline__ T inv_norm(const T * __restrict__ s, const int take_sqrt)
+        {
+            return T(1) / (take_sqrt ? sqrt(s[0]) : s[0]);
+        }
+        template <typename T>
+        __device__ __forceinline__ void multi_axpy_at(const int64_t i, const int64_t ldv, const int k1, const T * __restrict__ eta,
+                                                      const T * __restrict__ V, T * __restrict__ x)
+        {
+            T acc = x[i];
+            for (int k = 0; k < k1; ++k)
+                acc = eta[k] * V[i + (size_t)k * ldv] + acc;
+            x[i] = acc;
+        }
+
         template <typename T>
         __global__ void axpby_kernel(const int64_t n, const T a, const T * __restrict__ x, const T b, T * __restrict__ y)
         {
             const int64_t i = blockIdx.x * (int64_t)blockDim.x + threadIdx.x;
             if (i < n)
-                y[i] = a * x[i] + b * y[i];
+                axpby_at(i, a, x, b, y);
         }
         template <typename T>
         __global__ void scal_kernel(const int64_t n, const T a, T * __restrict__ x)
@@ -359,7 +397,7 @@ namespace cb200
         __global__ void scal_inv_dev_kernel(const int64_t n, const T * __restrict__ s, const int take_sqrt, T * __restrict__ x)
         {
             const int64_t i = blockIdx.x * (int64_t)blockDim.x + threadIdx.x;
-            const T a = T(1) / (take_sqrt ? sqrt(s[0]) : s[0]);
+            const T a = inv_norm(s, take_sqrt);
             if (i < n)
                 x[i] *= a;
         }
@@ -383,12 +421,8 @@ namespace cb200
                                           T * __restrict__ x)
         {
             const int64_t i = blockIdx.x * (int64_t)blockDim.x + threadIdx.x;
-            if (i >= n)
-                return;
-            T acc = x[i];
-            for (int k = 0; k < k1; ++k)
-                acc = eta[k] * V[i + (size_t)k * ldv] + acc;
-            x[i] = acc;
+            if (i < n)
+                multi_axpy_at(i, ldv, k1, eta, V, x);
         }
         // masked sum of squares / products in T (the residual norms of the distributed solve)
         template <typename T>
@@ -416,6 +450,71 @@ namespace cb200
         }
 
         inline unsigned nblk(int64_t n, int bs = 256) { return (unsigned)((n + bs - 1) / bs); }
+
+        // ---- batched solve (gmres_batch): grid row blockIdx.y = one active system, kernel arguments passed by value ----
+        template <typename T>
+        struct BatchArgs
+        {
+            const T * x[GMRES_BATCH_KMAX];
+            T * y[GMRES_BATCH_KMAX];
+            T a[GMRES_BATCH_KMAX], b[GMRES_BATCH_KMAX];
+            int k1[GMRES_BATCH_KMAX];  // multi_axpy: basis columns of each system
+            int sys[GMRES_BATCH_KMAX]; // system index: its slice of the basis, Hessenberg column, partials and ticket
+        };
+
+        template <typename T>
+        __global__ void axpby_batch_kernel(const int64_t n, const BatchArgs<T> p)
+        {
+            const int64_t i = blockIdx.x * (int64_t)blockDim.x + threadIdx.x;
+            const int j = blockIdx.y;
+            if (i < n)
+                axpby_at(i, p.a[j], p.x[j], p.b[j], p.y[j]);
+        }
+
+        // x_j += sum_k eta_j[k] V_j[:, k], eta_j at eta + sys * m1
+        template <typename T>
+        __global__ void multi_axpy_batch_kernel(const int64_t n, const int64_t ldv, const T * __restrict__ eta, const int m1, const BatchArgs<T> p)
+        {
+            const int64_t i = blockIdx.x * (int64_t)blockDim.x + threadIdx.x;
+            const int j = blockIdx.y;
+            if (i < n)
+                multi_axpy_at(i, ldv, p.k1[j], eta + (size_t)p.sys[j] * m1, p.x[j], p.y[j]);
+        }
+
+        // <x_j, x_j> -> result[j], each system with its own partials and ticket
+        template <typename T>
+        __global__ void __launch_bounds__(RED_THREADS)
+        norm2_batch_kernel(const int64_t n, T * __restrict__ partials, unsigned * __restrict__ tickets, T * __restrict__ result, const BatchArgs<T> p)
+        {
+            const int j = blockIdx.y, s = p.sys[j];
+            reduce_block<T, 0>(n, p.x[j], p.x[j], partials + (size_t)s * gridDim.x, tickets + s, result + j, 0);
+        }
+
+        // step j of the fused MGS sweep at Arnoldi index k1 - 1 for every listed system (basis of system s at V + s * vstride,
+        // Hessenberg column at H + s * hstride)
+        template <typename T>
+        __global__ void __launch_bounds__(RED_THREADS)
+        mgs_step_batch_kernel(const int64_t n, T * __restrict__ V, const int64_t ldv, const int64_t vstride, T * __restrict__ H, const int hstride,
+                              const int k1, const int jstep, T * __restrict__ partials, unsigned * __restrict__ tickets, const BatchArgs<T> p)
+        {
+            const int s = p.sys[blockIdx.y];
+            T * Vs = V + (size_t)s * vstride;
+            T * hs = H + (size_t)s * hstride;
+            mgs_step_block<T>(n, Vs + (size_t)k1 * ldv, jstep > 0 ? Vs + (size_t)(jstep - 1) * ldv : nullptr, jstep < k1 ? Vs + (size_t)jstep * ldv : nullptr,
+                              hs + (jstep > 0 ? jstep - 1 : 0), nullptr, partials + (size_t)s * gridDim.x, tickets + s, hs + jstep, jstep == k1 ? 1 : 0);
+        }
+
+        // w_s /= ||w_s|| (w_s = column k1 of system s, the norm at H[s * hstride + k1])
+        template <typename T>
+        __global__ void scal_inv_batch_kernel(const int64_t n, T * __restrict__ V, const int64_t ldv, const int64_t vstride, const T * __restrict__ H,
+                                              const int hstride, const int k1, const BatchArgs<T> p)
+        {
+            const int64_t i = blockIdx.x * (int64_t)blockDim.x + threadIdx.x;
+            const int s = p.sys[blockIdx.y];
+            const T a = inv_norm(H + (size_t)s * hstride + k1, 0);
+            if (i < n)
+                V[(size_t)s * vstride + (size_t)k1 * ldv + i] *= a;
+        }
 
         // reduction workspace of one thread of execution
         struct RedWork
@@ -845,6 +944,227 @@ namespace cb200
         out.num_iter = it;
         return out;
     }
+
+    // ---------------------------------------------------------------------------------------------
+    // Lockstep batched GMRES(m), MGS arithmetic: k independent gmres(..., ORTH_MGS) solves that share their launches. All active
+    // systems sit at the same Arnoldi index; every reduction of a system runs the single solve's kernel body on its own grid row
+    // with red_blocks(n) blocks, its own partials and ticket, so each system's results are bitwise those of its own solve.
+    // ---------------------------------------------------------------------------------------------
+    template <typename T>
+    std::vector<GmresResult> gmres_batch(int64_t n, int k, T * const * x, ApplyBatchFn<T> A, void * ctx, const T * const * b, int m, int maxit,
+                                         T tol, double max_seconds, cudaStream_t s)
+    {
+        NvtxRange nvtx_solve("cuddh::gmres_batch<float>");
+        CB_REQUIRE(k >= 1 && k <= GMRES_BATCH_KMAX, "gmres_batch: k must be in [1, " + std::to_string(GMRES_BATCH_KMAX) + "]");
+        CB_REQUIRE(x != nullptr && b != nullptr, "gmres_batch: null pointer array");
+        CB_REQUIRE(A != nullptr, "gmres_batch: null operator callback");
+        CB_REQUIRE(m >= 1, "gmres_batch: m must be >= 1");
+        CB_REQUIRE(n >= 0, "gmres_batch: negative size");
+        for (int j = 0; j < k; ++j) {
+            CB_REQUIRE(x[j] != nullptr && b[j] != nullptr, "gmres_batch: null vector pointer");
+            for (int i = 0; i < j; ++i)
+                CB_REQUIRE(x[j] + n <= x[i] || x[i] + n <= x[j], "gmres_batch: solution vectors " + std::to_string(i) + " and " + std::to_string(j) + " overlap");
+        }
+
+        std::vector<GmresResult> out((size_t)k);
+        for (auto & o : out) {
+            o.success = false;
+            o.num_iter = 0;
+            o.num_matvec = 0;
+        }
+        const T one = 1, zero = 0;
+        const int m1 = m + 1, hstride = m1 + 2;
+        const int64_t ldv = (n + 3) & ~int64_t(3), vstride = ldv * m1;
+        const int rb = red_blocks(n);
+
+        DevBuf<T> R_((size_t)ldv * k), V_((size_t)vstride * k), H_((size_t)hstride * k), part_((size_t)rb * k), res_((size_t)2 * k),
+            eta_((size_t)m1 * k);
+        DevBuf<unsigned> tick_((size_t)k);
+        CB_CUDA(cudaMemsetAsync(tick_.p, 0, sizeof(unsigned) * (size_t)k, s));
+        CB_CUDA(cudaMemsetAsync(V_.p, 0, sizeof(T) * (size_t)vstride * k, s));
+        auto Rv = [&](int j) { return R_.p + (size_t)j * ldv; };
+        auto Vv = [&](int j, int col) { return V_.p + (size_t)j * vstride + (size_t)col * ldv; };
+
+        // per-system host state of the single solve
+        std::vector<T> H((size_t)k * m1 * m, T(0)), sn((size_t)k * m, T(0)), cs((size_t)k * m, T(0)), eta((size_t)k * m1, T(0)),
+            hcol((size_t)k * hstride), hres((size_t)2 * k), bnrm(k), r_nrm(k);
+        std::vector<int> k1s(k, 0);
+
+        std::vector<const T *> ain;
+        std::vector<T *> aout;
+        // A on the listed systems, in[j] -> out[j]
+        auto apply = [&](const std::vector<int> & sys, auto in_of, auto out_of) {
+            ain.clear();
+            aout.clear();
+            for (int j : sys) {
+                ain.push_back(in_of(j));
+                aout.push_back(out_of(j));
+            }
+            const int rc = A(ctx, (int)sys.size(), ain.data(), aout.data(), s);
+            if (rc != 0)
+                throw Error(rc, std::string("gmres_batch: the operator callback failed (status ") + std::to_string(rc) + "): " + get_last_error());
+            for (int j : sys)
+                out[j].num_matvec++;
+        };
+        auto args_of = [&](const std::vector<int> & sys) {
+            BatchArgs<T> a{};
+            for (size_t i = 0; i < sys.size(); ++i)
+                a.sys[i] = sys[i];
+            return a;
+        };
+        // r_j = b_j - r_j
+        auto residual = [&](const std::vector<int> & sys) {
+            BatchArgs<T> a = args_of(sys);
+            for (size_t i = 0; i < sys.size(); ++i) {
+                a.x[i] = b[sys[i]];
+                a.y[i] = Rv(sys[i]);
+                a.a[i] = one;
+                a.b[i] = -one;
+            }
+            axpby_batch_kernel<T><<<dim3(nblk(n), (unsigned)sys.size()), 256, 0, s>>>(n, a);
+            CB_LAUNCHED();
+        };
+        // <v_j, v_j> of the listed systems -> res_[off + i]
+        auto norms2 = [&](const std::vector<int> & sys, auto vec_of, int off) {
+            BatchArgs<T> a = args_of(sys);
+            for (size_t i = 0; i < sys.size(); ++i)
+                a.x[i] = vec_of(sys[i]);
+            norm2_batch_kernel<T><<<dim3((unsigned)rb, (unsigned)sys.size()), RED_THREADS, 0, s>>>(n, part_.p, tick_.p, res_.p + off, a);
+            CB_LAUNCHED();
+        };
+        auto fetch = [&](T * dst, const T * src, size_t count) {
+            CB_CUDA(cudaMemcpyAsync(dst, src, sizeof(T) * count, cudaMemcpyDeviceToHost, s));
+            CB_CUDA(cudaStreamSynchronize(s));
+        };
+
+        std::vector<int> active(k);
+        for (int j = 0; j < k; ++j)
+            active[j] = j;
+        apply(active, [&](int j) { return (const T *)x[j]; }, Rv);
+        residual(active);
+        norms2(active, [&](int j) { return b[j]; }, 0);
+        norms2(active, [&](int j) { return (const T *)Rv(j); }, k);
+        fetch(hres.data(), res_.p, (size_t)2 * k);
+        {
+            std::vector<int> still;
+            for (int j = 0; j < k; ++j) {
+                bnrm[j] = (T)std::sqrt((double)hres[j]);
+                r_nrm[j] = (T)std::sqrt((double)hres[k + j]);
+                out[j].res_norm.push_back((double)r_nrm[j]);
+                out[j].time.push_back(0.0);
+                if (r_nrm[j] < tol * bnrm[j])
+                    out[j].success = true; // converged at the initial guess: 0 iterations
+                else
+                    still.push_back(j);
+            }
+            active.swap(still);
+        }
+        const auto t0 = std::chrono::high_resolution_clock::now();
+
+        int it = 1;
+        for (; it < maxit && !active.empty(); ++it) {
+            NvtxRange nvtx_cycle("gmres_batch restart cycle");
+            {
+                BatchArgs<T> a = args_of(active); // v0 = r / ||r||
+                for (size_t i = 0; i < active.size(); ++i) {
+                    const int j = active[i];
+                    a.x[i] = Rv(j);
+                    a.y[i] = Vv(j, 0);
+                    a.a[i] = one / r_nrm[j];
+                    a.b[i] = zero;
+                    std::fill(eta.begin() + (size_t)j * m1, eta.begin() + (size_t)(j + 1) * m1, T(0));
+                    eta[(size_t)j * m1] = r_nrm[j];
+                    k1s[j] = 0;
+                }
+                axpby_batch_kernel<T><<<dim3(nblk(n), (unsigned)active.size()), 256, 0, s>>>(n, a);
+                CB_LAUNCHED();
+            }
+
+            std::vector<int> inner = active; // systems still in this cycle's Arnoldi loop
+            for (int kk = 0; kk < m && !inner.empty(); ++kk) {
+                const int k1 = kk + 1;
+                for (int j : inner)
+                    k1s[j] = k1;
+                apply(inner, [&](int j) { return (const T *)Vv(j, kk); }, [&](int j) { return Vv(j, k1); });
+                const BatchArgs<T> a = args_of(inner);
+                const dim3 grid_red((unsigned)rb, (unsigned)inner.size()), grid_el(nblk(n), (unsigned)inner.size());
+                {
+                    NvtxRange nvtx_orth("gmres_batch orthogonalise (MGS)");
+                    for (int js = 0; js <= k1; ++js) {
+                        mgs_step_batch_kernel<T><<<grid_red, RED_THREADS, 0, s>>>(n, V_.p, ldv, vstride, H_.p, hstride, k1, js, part_.p, tick_.p, a);
+                        CB_LAUNCHED();
+                    }
+                    scal_inv_batch_kernel<T><<<grid_el, 256, 0, s>>>(n, V_.p, ldv, vstride, H_.p, hstride, k1, a);
+                    CB_LAUNCHED();
+                    fetch(hcol.data(), H_.p, (size_t)k * hstride);
+                }
+                std::vector<int> next;
+                for (int j : inner) {
+                    T * Hk = &H[(size_t)j * m1 * m + (size_t)m1 * kk];
+                    for (int i = 0; i <= k1; ++i)
+                        Hk[i] = hcol[(size_t)j * hstride + i];
+                    if (Hk[k1] == T(0)) { // w was all zeros: undo the 0/0 scaling and wait for the restart
+                        CB_CUDA(cudaMemsetAsync(Vv(j, k1), 0, sizeof(T) * (size_t)n, s));
+                        continue;
+                    }
+                    T * e = &eta[(size_t)j * m1];
+                    T * c = &cs[(size_t)j * m];
+                    T * sg = &sn[(size_t)j * m];
+                    givens(Hk, c, sg, kk);
+                    e[k1] = -sg[kk] * e[kk];
+                    e[kk] = c[kk] * e[kk];
+                    if (std::abs(e[k1]) < tol * bnrm[j])
+                        continue;
+                    next.push_back(j);
+                }
+                inner.swap(next);
+            }
+
+            // restart tail: x += V eta, true residual
+            for (int j : active)
+                trsv_upper<T>(k1s[j], &H[(size_t)j * m1 * m], m1, &eta[(size_t)j * m1]);
+            CB_CUDA(cudaMemcpyAsync(eta_.p, eta.data(), sizeof(T) * eta.size(), cudaMemcpyHostToDevice, s));
+            {
+                BatchArgs<T> a = args_of(active);
+                for (size_t i = 0; i < active.size(); ++i) {
+                    const int j = active[i];
+                    a.x[i] = Vv(j, 0);
+                    a.y[i] = x[j];
+                    a.k1[i] = k1s[j];
+                }
+                multi_axpy_batch_kernel<T><<<dim3(nblk(n), (unsigned)active.size()), 256, 0, s>>>(n, ldv, eta_.p, m1, a);
+                CB_LAUNCHED();
+            }
+            apply(active, [&](int j) { return (const T *)x[j]; }, Rv);
+            residual(active);
+            norms2(active, [&](int j) { return (const T *)Rv(j); }, 0);
+            fetch(hres.data(), res_.p, active.size());
+            const auto t1 = std::chrono::high_resolution_clock::now();
+            const double dur = 1e-9 * std::chrono::duration_cast<std::chrono::nanoseconds>(t1 - t0).count();
+            std::vector<int> still;
+            for (size_t i = 0; i < active.size(); ++i) {
+                const int j = active[i];
+                r_nrm[j] = (T)std::sqrt((double)hres[i]);
+                out[j].res_norm.push_back((double)r_nrm[j]);
+                out[j].time.push_back(dur);
+                if (dur > max_seconds)
+                    out[j].num_iter = it;
+                else if (r_nrm[j] < tol * bnrm[j]) {
+                    out[j].success = true;
+                    out[j].num_iter = it;
+                }
+                else
+                    still.push_back(j);
+            }
+            active.swap(still);
+        }
+        for (int j : active)
+            out[j].num_iter = it;
+        return out;
+    }
+
+    template std::vector<GmresResult> gmres_batch<float>(int64_t, int, float * const *, ApplyBatchFn<float>, void *, const float * const *, int, int,
+                                                         float, double, cudaStream_t);
 
     template GmresResult gmres<double>(int64_t, double *, ApplyFn<double>, void *, const double *, int, int, double, int, double, cudaStream_t,
                                        const GmresOptions &);

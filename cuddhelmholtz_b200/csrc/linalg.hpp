@@ -51,6 +51,21 @@ namespace cb200
     GmresResult gmres(int64_t n, T * x, ApplyFn<T> A, void * ctx, const T * b, int m, int maxit, T tol, int verbose,
                       double max_seconds, cudaStream_t s, const GmresOptions & opt = GmresOptions());
 
+    // y_j = A x_j for the k systems listed, enqueued on stream s (x, y: HOST arrays of k device pointers); non-zero aborts the solve
+    template <typename T> using ApplyBatchFn = int (*)(void * ctx, int k, const T * const * x, T * const * y, cudaStream_t s);
+    constexpr int GMRES_BATCH_KMAX = 32;
+
+    // k (<= GMRES_BATCH_KMAX) independent GMRES(m) solves A x_j = b_j in lockstep: every Arnoldi step applies A once to all systems
+    // still in their Arnoldi loop (A is handed only those), runs their MGS sweeps in the same launches and syncs the host once.
+    // Each system keeps the control flow of gmres(..., ORTH_MGS): its own initial-residual exit, inner break (|eta| < tol ||b||
+    // or w = 0; it then waits for the restart boundary), true residual per restart, and it leaves the batch when it converges.
+    // Results (x, res_norm, num_iter, num_matvec) are bitwise those of k sequential gmres(..., ORTH_MGS) calls; time[] is measured
+    // from the start of the batch, and max_seconds limits the wall time of the whole batch. MGS only (GmresOptions::orth is not
+    // read); no CGS2, distributed vectors, preconditioning or verbose output. Only float is instantiated.
+    template <typename T>
+    std::vector<GmresResult> gmres_batch(int64_t n, int k, T * const * x, ApplyBatchFn<T> A, void * ctx, const T * const * b, int m, int maxit,
+                                         T tol, double max_seconds, cudaStream_t s);
+
     // process-wide default of GmresOptions::orth for the entry points without an options argument (set_option "gmres_orth")
     int default_gmres_orth();
     void set_default_gmres_orth(int v);

@@ -339,6 +339,26 @@ int cuddh_b200_ddh_transfer_info(cuddh_ddh_transfer_t h, int64_t * info);
 /* host copy of M_dom: (2F, 2F) column-major floats */
 int cuddh_b200_ddh_transfer_get_block(cuddh_ddh_transfer_t h, int dom, float * h_out);
 
+/* ---- many right-hand sides at once (new) -------------------------------------------------------------------------------
+ * Batched operator callback: must enqueue y[j] = A x[j] for j < k on `stream` and return 0. x, y: HOST arrays of k DEVICE
+ * pointers; a non-zero return aborts the solve, which then returns that status. */
+typedef int (*cuddh_apply_batch_f_fn)(void * ctx, int k, const float * const * x, float * const * y, void * stream);
+/* y[j] = x[j] - T x[j] for j < k, 1 <= k <= 32. Row j is bitwise cuddh_b200_ddh_transfer_action(x[j]); the blocks are streamed once
+ * for up to 16 vectors (ceil(k / 16) launches). Fails if any y[j] overlaps any x[i] or another y[i] (n = DDH::size() floats each). */
+int cuddh_b200_ddh_transfer_action_batch(cuddh_ddh_transfer_t h, int k, const float * const * x, float * const * y, void * stream);
+int cuddh_b200_ddh_transfer_as_apply_batch(void * transfer_handle, int k, const float * const * x, float * const * y,
+                                           void * stream); /* cuddh_apply_batch_f_fn */
+/* k (1 <= k <= 32) independent FP32 GMRES(m) solves A x[j] = b[j] in lockstep: each Arnoldi step applies A once to the systems still
+ * iterating (A is handed only those), orthogonalises them in the same launches and syncs the host once. Modified Gram-Schmidt
+ * only (the "gmres_orth" option is not read); no preconditioner, distributed vectors or verbose output. Each system follows the
+ * control flow of cuddh_b200_gmres_f with orth 0 and leaves the batch when it converges: its x, residual norms, num_iter and
+ * num_matvec are bitwise those of that solve. max_seconds limits the wall time of the whole batch; h_time is measured from its
+ * start. x, b: HOST arrays of k device pointers (the x[j] must not overlap). out: k entries or NULL; h_res_norm / h_time: HOST
+ * arrays of k * cap doubles (row j at j * cap) or NULL. */
+int cuddh_b200_gmres_f_batch(int64_t n, int k, float * const * x, cuddh_apply_batch_f_fn A, void * A_ctx, const float * const * b, int m,
+                             int maxit, float tol, double max_seconds, cuddh_solver_out * out, double * h_res_norm, double * h_time,
+                             int cap, void * stream);
+
 #ifdef __cplusplus
 }
 #endif
